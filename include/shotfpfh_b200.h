@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SF_ABI_VERSION 11
+#define SF_ABI_VERSION 12
 
 #define SF_OK 0
 #define SF_ERR_CUDA 1     /* a CUDA runtime call or kernel launch failed */
@@ -124,6 +124,26 @@ int sf_knn(sf_grid* grid, const double* queries_dev, int64_t nq, int32_t k, doub
  * normals_dev: float64 (nq,3); NaN for an empty neighbourhood, as NumPy gives. */
 int sf_pca_normals(const double* xyz_dev, int64_t nq, const int64_t* offsets_dev, int32_t fixed_k,
                    const int32_t* nbr_index_dev, const double* pre_normals_dev, double* normals_dev, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------
+ * K — salient keypoints (no counterpart in the reference). ISS, Intrinsic Shape Signatures (Zhong 2009), as Open3D
+ * defines it, with the covariance accumulated about the point; oracle/iss_oracle.py is the specification. Both calls
+ * take a grid built (sf_grid_build, normals not needed) for max(salient radius, non-max radius); each radius must be
+ * positive and within the grid's cell edge. Neighbourhoods use the fixed-radius predicate above.
+ * ---------------------------------------------------------------------------------------------------------- */
+/* saliency_dev: float64[n] per CELL-SORTED position: s_i = e3 of the covariance of the points within salient_radius
+ * (about their barycentre) where that neighbourhood holds >= min_neighbors points and e2/e1 < gamma_21 and
+ * e3/e2 < gamma_32 (e3 <= e2 <= e1, np.linalg.eigh's values), else 0. counts_dev (int32[n], the neighbourhood sizes)
+ * and eigvals_dev (float64 (n,3), ascending) may be NULL. min_neighbors >= 1, finite gammas.
+ * An empty handle (n = 0) writes nothing. No synchronisation. */
+int sf_iss_saliency(sf_grid* grid, double salient_radius, int32_t min_neighbors, double gamma_21, double gamma_32,
+                    double* saliency_dev, int32_t* counts_dev, double* eigvals_dev, void* stream);
+/* Non-maximum suppression: point i is a keypoint iff s_i > 0, at least min_neighbors points lie within
+ * non_max_radius of it, and none of them has a larger saliency (ties keep both). keypoints_dev: int32[n] capacity;
+ * the first *count_host entries receive the keypoints' ORIGINAL indices in ascending order. Synchronises `stream`
+ * (the count is a host result); *count_host = 0 for an empty handle. */
+int sf_iss_select(sf_grid* grid, const double* saliency_dev, double non_max_radius, int32_t min_neighbors,
+                  int32_t* keypoints_dev, int64_t* count_host, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * S — SHOT.

@@ -4,8 +4,10 @@ compute_descriptors, find_descriptors_matches, run_ransac, run_icp) through THIS
 NumPy arrays in and out at every stage, on a synthetic rigid pair (SURVEY.md 8d generator). BASELINE.json configs[4]
 names a 10M-point pair; the size is an argument:
 
-    python scripts/run_registration_flow.py [n_points] [fpfh]
+    python scripts/run_registration_flow.py [n_points] [fpfh] [voxel|iss]
 
+The keypoint selector is `voxel` (select_keypoints_subsampling, 3.75 spacings: the default) or `iss`
+(select_keypoints_iss, salient radius 5 spacings, non-max radius 3.75 spacings: far fewer keypoints, on salient points).
 Prints wall-clock per stage and the error of the recovered transform against the known one. (`/root/reference` is not
 on the GPU box, so its `RegistrationPipeline` object cannot be run there; `dropin.install()` binds exactly these
 callables into it.)
@@ -24,11 +26,11 @@ from shot_fpfh_b200 import synthetic  # noqa: E402
 from shot_fpfh_b200.core import RigidTransform  # noqa: E402
 from shot_fpfh_b200.descriptors import ShotMultiprocessor, compute_fpfh_descriptor  # noqa: E402
 from shot_fpfh_b200.icp import icp_point_to_plane  # noqa: E402
-from shot_fpfh_b200.keypoint_selection import select_keypoints_subsampling  # noqa: E402
+from shot_fpfh_b200.keypoint_selection import select_keypoints_iss, select_keypoints_subsampling  # noqa: E402
 from shot_fpfh_b200.matching import match_descriptors, ransac_on_matches  # noqa: E402
 
 
-def run(n: int, with_fpfh: bool = False, verbose: bool = True) -> dict:
+def run(n: int, with_fpfh: bool = False, verbose: bool = True, keypoints: str = "voxel") -> dict:
     times = {}
 
     def stage(name, fn):
@@ -48,8 +50,14 @@ def run(n: int, with_fpfh: bool = False, verbose: bool = True) -> dict:
     radius = 5.0 * s
     if verbose:
         print(f"pair of {n} points, radius {radius:.5f}")
-    scan_kp = stage("select_keypoints (scan)", lambda: select_keypoints_subsampling(scan, 3.75 * s))
-    ref_kp = stage("select_keypoints (ref)", lambda: select_keypoints_subsampling(ref, 3.75 * s))
+    if keypoints == "iss":
+        select = lambda cloud: select_keypoints_iss(cloud, 5.0 * s, 3.75 * s)  # noqa: E731
+    elif keypoints == "voxel":
+        select = lambda cloud: select_keypoints_subsampling(cloud, 3.75 * s)  # noqa: E731
+    else:
+        raise ValueError(f"unknown keypoint selector {keypoints!r} (voxel or iss)")
+    scan_kp = stage(f"select_keypoints {keypoints} (scan)", lambda: select(scan))
+    ref_kp = stage(f"select_keypoints {keypoints} (ref)", lambda: select(ref))
     with ShotMultiprocessor(min_neighborhood_size=10, verbose=False) as shot:
         scan_desc = stage("SHOT single scale (scan)", lambda: shot.compute_descriptor_single_scale(
             scan, normals, scan[scan_kp], radius))
@@ -72,7 +80,7 @@ def run(n: int, with_fpfh: bool = False, verbose: bool = True) -> dict:
         scan, ref, ref_normals, RigidTransform(coarse.rotation, coarse.translation), d_max=2 * s, voxel_size=3.75 * s,
         max_iter=20, rms_threshold=1e-9))
     out = {
-        "n_points": n, "keypoints": (int(scan_kp.shape[0]), int(ref_kp.shape[0])), "matches": int(matches[0].shape[0]),
+        "n_points": n, "keypoint_selector": keypoints, "keypoints": (int(scan_kp.shape[0]), int(ref_kp.shape[0])), "matches": int(matches[0].shape[0]),
         "ransac_inlier_ratio": float(ratio),
         "coarse_rotation_error": float(np.abs(coarse.rotation - rot).max()),
         "fine_rotation_error": float(np.abs(fine.rotation - rot).max()),
@@ -87,4 +95,5 @@ def run(n: int, with_fpfh: bool = False, verbose: bool = True) -> dict:
 
 if __name__ == "__main__":
     size = int(sys.argv[1]) if len(sys.argv) > 1 else 10_000_000
-    run(size, with_fpfh=len(sys.argv) > 2 and sys.argv[2] == "fpfh")
+    words = sys.argv[2:]
+    run(size, with_fpfh="fpfh" in words, keypoints="iss" if "iss" in words else "voxel")

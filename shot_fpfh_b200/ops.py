@@ -112,6 +112,32 @@ def pca_normals(xyz: torch.Tensor, nq: int, nbr_index: torch.Tensor, offsets: to
     return out
 
 
+def iss_saliency(grid: Grid, salient_radius: float, min_neighbors: int, gamma_21: float, gamma_32: float,
+                 want_counts: bool = False, want_eigvals: bool = False):
+    """
+    ISS saliency of every cloud point (sf_iss_saliency), in CELL-SORTED order (`grid_permutation` maps it to original
+    order). Returns (saliency float64 (n,), counts int32 (n,) | None, eigenvalues float64 (n, 3) ascending | None).
+    """
+    dev = require_cuda()
+    n = grid.n
+    sal = torch.empty(n, dtype=torch.float64, device=dev)
+    counts = torch.empty(n, dtype=torch.int32, device=dev) if want_counts else None
+    eig = torch.empty((n, 3), dtype=torch.float64, device=dev) if want_eigvals else None
+    check(lib.sf_iss_saliency(grid.handle, float(salient_radius), int(min_neighbors), float(gamma_21), float(gamma_32),
+                              ptr(sal), ptr(counts), ptr(eig), stream_ptr()))
+    return sal, counts, eig
+
+
+def iss_select(grid: Grid, saliency: torch.Tensor, non_max_radius: float, min_neighbors: int) -> torch.Tensor:
+    """Non-maximum suppression of the cell-sorted `saliency` (sf_iss_select) -> int64 original indices, ascending."""
+    dev = require_cuda()
+    out = torch.empty(max(grid.n, 1), dtype=torch.int32, device=dev)
+    count = ctypes.c_int64(0)
+    check(lib.sf_iss_select(grid.handle, ptr(saliency), float(non_max_radius), int(min_neighbors), ptr(out),
+                            ctypes.byref(count), stream_ptr()))
+    return out[: int(count.value)].long()
+
+
 def shot_lrf(grid: Grid, queries: torch.Tensor, radius: float, offsets: torch.Tensor, nbr_sorted: torch.Tensor):
     nq = int(queries.shape[0])
     lrf = torch.empty((nq, 3, 3), dtype=torch.float64, device=queries.device)
