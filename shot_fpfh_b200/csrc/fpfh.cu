@@ -462,6 +462,15 @@ __global__ void __launch_bounds__(256)
 
 using namespace sf;
 
+// Floats per SPFH row: 3 n_bins (decorrelated) or n_bins^3, with n_bins in [1, kMaxBins] and at most 8192 bins.
+static int histogram_width(const char* who, int32_t n_bins, int32_t decorrelated, int* width) {
+  SF_REQUIRE(n_bins >= 1 && n_bins <= kMaxBins, SF_ERR_CAPACITY, "%s: n_bins must be in [1, %d]", who, kMaxBins);
+  const int64_t width64 = decorrelated ? 3 * int64_t(n_bins) : int64_t(n_bins) * n_bins * n_bins;
+  SF_REQUIRE(width64 <= 8192, SF_ERR_CAPACITY, "%s: histogram width %lld exceeds 8192", who, (long long)width64);
+  *width = int(width64);
+  return SF_OK;
+}
+
 static int launch_spfh(sf_grid* g, int64_t first, int64_t count, const int64_t* offsets, const int32_t* counts,
                        const int32_t* nbr, int32_t n_bins, int32_t decorrelated, const double* edges_host, float* spfh,
                        int stride, cudaStream_t stream) {
@@ -469,10 +478,8 @@ static int launch_spfh(sf_grid* g, int64_t first, int64_t count, const int64_t* 
   SF_REQUIRE(offsets && nbr && edges_host && spfh, SF_ERR_ARG, "sf_spfh: null argument");
   SF_REQUIRE(first >= 0 && count >= 0 && first + count <= g->n, SF_ERR_ARG, "sf_spfh: point range outside the cloud");
   if (count == 0) return SF_OK;
-  SF_REQUIRE(n_bins >= 1 && n_bins <= kMaxBins, SF_ERR_CAPACITY, "sf_spfh: n_bins must be in [1, %d]", kMaxBins);
-  const int64_t width64 = decorrelated ? 3 * int64_t(n_bins) : int64_t(n_bins) * n_bins * n_bins;
-  SF_REQUIRE(width64 <= 8192, SF_ERR_CAPACITY, "sf_spfh: histogram width %lld exceeds 8192", (long long)width64);
-  const int width = int(width64);
+  int width = 0;
+  if (int rc = histogram_width("sf_spfh", n_bins, decorrelated, &width)) return rc;
   double edges[3][kMaxBins + 1] = {};
   for (int f = 0; f < 3; ++f)
     for (int b = 0; b <= n_bins; ++b) edges[f][b] = edges_host[f * (n_bins + 1) + b];
@@ -532,16 +539,17 @@ static int launch_fpfh(sf_grid* g, const int64_t* offsets, const int32_t* counts
   // processing order: keypoints by cell-sorted position (see fpfh_kernel); not worth a sort for a handful
   int32_t *pos = nullptr, *ids = nullptr, *pos_sorted = nullptr, *order = nullptr;
   void* sort_temp = nullptr;
+  Scratch scratch(stream);
   if (nq >= 4096 && nq < (int64_t(1) << 31)) {
     size_t sort_bytes = 0;
     int end_bit = 1;
     while ((int64_t(1) << end_bit) < g->n) ++end_bit;
     cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, pos, pos_sorted, ids, order, int(nq), 0, end_bit, stream);
-    SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&pos), size_t(nq) * 4, stream));
-    SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&ids), size_t(nq) * 4, stream));
-    SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&pos_sorted), size_t(nq) * 4, stream));
-    SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&order), size_t(nq) * 4, stream));
-    SF_CUDA(scratch_alloc(&sort_temp, sort_bytes + 16, stream));
+    SF_CUDA(scratch.alloc(&pos, size_t(nq) * 4));
+    SF_CUDA(scratch.alloc(&ids, size_t(nq) * 4));
+    SF_CUDA(scratch.alloc(&pos_sorted, size_t(nq) * 4));
+    SF_CUDA(scratch.alloc(&order, size_t(nq) * 4));
+    SF_CUDA(scratch.alloc(&sort_temp, sort_bytes + 16));
     keypoint_position_kernel<<<unsigned((nq + 255) / 256), 256, 0, stream>>>(g->inv_perm, keypoints, nq, pos, ids);
     SF_CUDA(cub::DeviceRadixSort::SortPairs(sort_temp, sort_bytes, pos, pos_sorted, ids, order, int(nq), 0, end_bit,
                                             stream));
@@ -560,9 +568,6 @@ static int launch_fpfh(sf_grid* g, const int64_t* offsets, const int32_t* counts
       default: set_error("fpfh: padded stride %d unsupported", stride); return SF_ERR_ARG;
     }
 #undef SF_LAUNCH_ROWS4
-    void* to_free4[] = {pos, ids, pos_sorted, order, sort_temp};
-    for (void* p : to_free4)
-      if (p) cudaFreeAsync(p, stream);
     SF_CUDA(cudaGetLastError());
     return SF_OK;
   }
@@ -589,9 +594,6 @@ static int launch_fpfh(sf_grid* g, const int64_t* offsets, const int32_t* counts
 #undef SF_LAUNCH_FPFH
     base += blocks_n * 32 + rem;
   }
-  void* to_free[] = {pos, ids, pos_sorted, order, sort_temp};
-  for (void* p : to_free)
-    if (p) cudaFreeAsync(p, stream);
   SF_CUDA(cudaGetLastError());
   return SF_OK;
 }
@@ -609,100 +611,111 @@ extern "C" int sf_fpfh(sf_grid* g, const int64_t* offsets, const int32_t* nbr, c
                                   nq, 0, static_cast<float*>(out), stream);
 }
 
-// Fused driver: what compute_fpfh_descriptor (fpfh.py:16-117) does for one cloud — search around EVERY cloud point,
-// SPFH of every point, FPFH of the keypoints — with the neighbour list as an internal, padded temporary.
+// ---- the fused drivers: four stages on the cell-sorted points [first, first + count) ----------------------------------
+//   candidates  padded list offsets (fpfh_candidates)                             sf_fpfh_block_begin
+//   search      padded neighbour lists, weights 1 / d, counts (fpfh_search)       sf_fpfh_block_spfh
+//   SPFH        rows of `stride` floats (launch_spfh)                             sf_fpfh_block_spfh
+//   (multi-GPU caller: all-gather of the blocks' SPFH rows)
+//   rows        FPFH rows of the keypoints in the block (launch_fpfh)             sf_fpfh_block_rows
+// sf_fpfh_cloud runs the four on the whole cloud with its own temporaries; the block entry points run them on one block
+// per GPU, and the temporaries between them belong to the caller.
+
+// SPFH rows of up to 128 bins are padded to a multiple of four floats for fpfh_rows4_kernel (SF_FPFH_NO_ROWS4=1:
+// measurement / test switch back to the per-neighbour gather of fpfh_kernel, on unpadded rows).
+static void fpfh_row_layout(int width, int* stride, int* rows4) {
+  const char* no_rows4 = getenv("SF_FPFH_NO_ROWS4");
+  *rows4 = (width <= 128 && !(no_rows4 != nullptr && no_rows4[0] == '1')) ? 1 : 0;
+  *stride = *rows4 ? (width + 3) / 4 * 4 : width;
+}
+
+// count > 0; reads *total = cand_offsets[count] back (synchronises the stream)
+static int fpfh_candidates(sf_grid* g, int64_t first, int64_t count, int64_t* cand_offsets, int64_t* total,
+                           Scratch& scratch, cudaStream_t stream) {
+  int64_t* cand = nullptr;
+  void* scan_temp = nullptr;
+  size_t scan_bytes = 0;
+  cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, cand, cand_offsets, int(count + 1), stream);
+  SF_CUDA(scratch.alloc(&cand, size_t(count + 1) * 8));
+  SF_CUDA(scratch.alloc(&scan_temp, scan_bytes + 16));
+  SF_CUDA(cudaMemsetAsync(cand + count, 0, 8, stream));
+  self_candidate_count_kernel<<<unsigned((count + 255) / 256), 256, 0, stream>>>(g->view(), first, count, cand);
+  SF_CUDA(cub::DeviceScan::ExclusiveSum(scan_temp, scan_bytes, cand, cand_offsets, int(count + 1), stream));
+  SF_CUDA(cudaMemcpyAsync(total, cand_offsets + count, 8, cudaMemcpyDeviceToHost, stream));
+  SF_CUDA(cudaStreamSynchronize(stream));
+  return SF_OK;
+}
+
+// adds the number of neighbour pairs to *pair_counter (zeroed by the caller)
+static int fpfh_search(sf_grid* g, double radius, int64_t first, int64_t count, const int64_t* cand_offsets,
+                       int32_t* nbr, float* weights, int32_t* counts, unsigned long long* pair_counter,
+                       cudaStream_t stream) {
+  const size_t smem = size_t(kSearchWarps) * sizeof(SearchStage);
+  static bool configured = false;
+  if (!configured) {
+    SF_CUDA(cudaFuncSetAttribute(search_weights_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    configured = true;
+  }
+  const int64_t tiles = (count + 31) / 32;
+  search_weights_kernel<<<unsigned((tiles + kSearchWarps - 1) / kSearchWarps), kSearchWarps * 32, smem, stream>>>(
+      g->view(), first, count, radius * radius, cand_offsets, nbr, weights, counts, pair_counter);
+  SF_CUDA(cudaGetLastError());
+  return SF_OK;
+}
+
+// synchronises the stream
+static int read_pairs(const unsigned long long* pair_counter, int64_t* pairs_host, cudaStream_t stream) {
+  unsigned long long pairs = 0;
+  SF_CUDA(cudaMemcpyAsync(&pairs, pair_counter, 8, cudaMemcpyDeviceToHost, stream));
+  SF_CUDA(cudaStreamSynchronize(stream));
+  *pairs_host = int64_t(pairs);
+  return SF_OK;
+}
+
+// What compute_fpfh_descriptor (fpfh.py:16-117) does for one cloud — search around EVERY cloud point, SPFH of every
+// point, FPFH of the keypoints — with the neighbour list as an internal, padded temporary.
 extern "C" int sf_fpfh_cloud(sf_grid* g, double radius, int32_t n_bins, int32_t decorrelated, const double* edges_host,
                              const int64_t* keypoints, int64_t nq, void* out, int32_t out_is_f64, int64_t* pairs_host,
                              void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   SF_REQUIRE(g != nullptr && g->n > 0 && g->has_normals, SF_ERR_ARG, "sf_fpfh_cloud: grid built without normals");
   SF_REQUIRE(edges_host && (nq == 0 || (keypoints && out)) && nq >= 0, SF_ERR_ARG, "sf_fpfh_cloud: bad arguments");
-  SF_REQUIRE(radius > 0.0 && radius * 1.0005 <= g->cell, SF_ERR_ARG,
+  SF_REQUIRE(radius_fits(g, radius), SF_ERR_ARG,
              "sf_fpfh_cloud: radius %g exceeds the cell edge %g the grid was built for", radius, g->cell);
-  SF_REQUIRE(n_bins >= 1 && n_bins <= kMaxBins, SF_ERR_CAPACITY, "sf_fpfh_cloud: n_bins must be in [1, %d]", kMaxBins);
-  const int64_t width64 = decorrelated ? 3 * int64_t(n_bins) : int64_t(n_bins) * n_bins * n_bins;
-  SF_REQUIRE(width64 <= 8192, SF_ERR_CAPACITY, "sf_fpfh_cloud: histogram width %lld exceeds 8192", (long long)width64);
-  const int width = int(width64);
+  int width = 0, stride = 0, rows4 = 0;
+  if (int rc = histogram_width("sf_fpfh_cloud", n_bins, decorrelated, &width)) return rc;
+  fpfh_row_layout(width, &stride, &rows4);
   const int64_t n = g->n;
   if (pairs_host) *pairs_host = 0;
-  int64_t *cand = nullptr, *cand_offsets = nullptr;
+  Scratch scratch(stream);
+  int64_t* cand_offsets = nullptr;
+  int64_t total = 0;
+  SF_CUDA(scratch.alloc(&cand_offsets, size_t(n + 1) * 8));
+  if (int rc = fpfh_candidates(g, 0, n, cand_offsets, &total, scratch, stream)) return rc;
   int32_t *counts = nullptr, *nbr = nullptr;
   float *weights = nullptr, *spfh = nullptr;
   unsigned long long* pair_counter = nullptr;
-  void* scan_temp = nullptr;
-  size_t scan_bytes = 0;
-  cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, cand, cand_offsets, int(n + 1), stream);
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&cand), size_t(n + 1) * 8, stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&cand_offsets), size_t(n + 1) * 8, stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&counts), size_t(n) * 4, stream));
-  SF_CUDA(scratch_alloc(&scan_temp, scan_bytes + 16, stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&pair_counter), 8, stream));
-  // rows of up to 128 bins are padded to a multiple of four floats for fpfh_rows4_kernel (SF_FPFH_NO_ROWS4=1:
-  // measurement / test switch back to the per-neighbour gather of fpfh_kernel)
-  const char* no_rows4 = getenv("SF_FPFH_NO_ROWS4");
-  const int rows4 = (width <= 128 && !(no_rows4 != nullptr && no_rows4[0] == '1')) ? 1 : 0;
-  const int stride = rows4 ? (width + 3) / 4 * 4 : width;
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&spfh), size_t(n) * stride * sizeof(float), stream));
-  SF_CUDA(cudaMemsetAsync(cand + n, 0, 8, stream));
+  SF_CUDA(scratch.alloc(&counts, size_t(n) * 4));
+  SF_CUDA(scratch.alloc(&pair_counter, 8));
+  SF_CUDA(scratch.alloc(&spfh, size_t(n) * stride * sizeof(float)));
+  SF_CUDA(scratch.alloc(&nbr, size_t(total > 0 ? total : 1) * 4));
+  SF_CUDA(scratch.alloc(&weights, size_t(total > 0 ? total : 1) * 4));
   SF_CUDA(cudaMemsetAsync(pair_counter, 0, 8, stream));
-  const GridView view = g->view();
-  self_candidate_count_kernel<<<unsigned((n + 255) / 256), 256, 0, stream>>>(view, 0, n, cand);
-  SF_CUDA(cub::DeviceScan::ExclusiveSum(scan_temp, scan_bytes, cand, cand_offsets, int(n + 1), stream));
-  int64_t total = 0;
-  SF_CUDA(cudaMemcpyAsync(&total, cand_offsets + n, 8, cudaMemcpyDeviceToHost, stream));
-  SF_CUDA(cudaStreamSynchronize(stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&nbr), size_t(total > 0 ? total : 1) * 4, stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&weights), size_t(total > 0 ? total : 1) * 4, stream));
   profile_mark(0, stream);
-  {
-    const size_t smem = size_t(kSearchWarps) * sizeof(SearchStage);
-    static bool configured = false;
-    if (!configured) {
-      SF_CUDA(cudaFuncSetAttribute(search_weights_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-      configured = true;
-    }
-    const int64_t tiles = (n + 31) / 32;
-    search_weights_kernel<<<unsigned((tiles + kSearchWarps - 1) / kSearchWarps), kSearchWarps * 32, smem, stream>>>(
-        view, 0, n, radius * radius, cand_offsets, nbr, weights, counts, pair_counter);
-  }
-  SF_CUDA(cudaGetLastError());
+  if (int rc = fpfh_search(g, radius, 0, n, cand_offsets, nbr, weights, counts, pair_counter, stream)) return rc;
   profile_mark(1, stream);
-  int rc = launch_spfh(g, 0, n, cand_offsets, counts, nbr, n_bins, decorrelated, edges_host, spfh, stride, stream);
+  if (int rc = launch_spfh(g, 0, n, cand_offsets, counts, nbr, n_bins, decorrelated, edges_host, spfh, stride, stream))
+    return rc;
   profile_mark(2, stream);
-  if (rc == SF_OK && nq > 0)
-    rc = out_is_f64 ? launch_fpfh(g, cand_offsets, counts, nbr, nullptr, weights, 0, spfh, width, stride, rows4, keypoints,
-                                  nq, 0, static_cast<double*>(out), stream)
-                    : launch_fpfh(g, cand_offsets, counts, nbr, nullptr, weights, 0, spfh, width, stride, rows4, keypoints,
-                                  nq, 0, static_cast<float*>(out), stream);
+  if (int rc = sf_fpfh_block_rows(g, 0, n, cand_offsets, counts, nbr, weights, spfh, width, keypoints, nq, out, out_is_f64,
+                                  stream))
+    return rc;
   profile_mark(3, stream);
-  if (rc == SF_OK && pairs_host != nullptr) {
-    unsigned long long pairs = 0;
-    SF_CUDA(cudaMemcpyAsync(&pairs, pair_counter, 8, cudaMemcpyDeviceToHost, stream));
-    SF_CUDA(cudaStreamSynchronize(stream));
-    *pairs_host = int64_t(pairs);
-  }
-  void* to_free[] = {cand, cand_offsets, counts, nbr, weights, spfh, scan_temp, pair_counter};
-  for (void* p : to_free)
-    if (p) cudaFreeAsync(p, stream);
-  return rc;
-}
-
-// ---- the fused driver by BLOCKS of the cell-sorted cloud (multi-GPU: one block per rank) ---------------------------------
-// The same three stages as sf_fpfh_cloud with the all-gather of the SPFH rows between the second and the third, so the
-// temporaries belong to the caller:
-//   sf_fpfh_block_begin  padded list offsets of the cell-sorted points [first, first + count)  -> total list length
-//   sf_fpfh_block_spfh   one scan of the candidates writes lists, weights, counts; SPFH rows of the block (stride floats)
-//   (caller: all-gather of the blocks' SPFH rows)
-//   sf_fpfh_block_rows   FPFH rows of the keypoints whose cell-sorted position lies in the block
-static int fpfh_row_layout(int width, int* stride, int* rows4) {
-  *rows4 = width <= 128 ? 1 : 0;
-  *stride = *rows4 ? (width + 3) / 4 * 4 : width;
-  return SF_OK;
+  return pairs_host != nullptr ? read_pairs(pair_counter, pairs_host, stream) : SF_OK;
 }
 
 extern "C" int sf_fpfh_row_stride(int32_t width, int32_t* stride_out) {
-  int stride = 0, rows4 = 0;
   SF_REQUIRE(width > 0 && stride_out != nullptr, SF_ERR_ARG, "sf_fpfh_row_stride: bad arguments");
+  int stride = 0, rows4 = 0;
   fpfh_row_layout(width, &stride, &rows4);
   *stride_out = stride;
   return SF_OK;
@@ -714,27 +727,15 @@ extern "C" int sf_fpfh_block_begin(sf_grid* g, double radius, int64_t first, int
   SF_REQUIRE(g != nullptr && g->n > 0, SF_ERR_ARG, "sf_fpfh_block_begin: grid not built");
   SF_REQUIRE(first >= 0 && count >= 0 && first + count <= g->n && cand_offsets && total_host, SF_ERR_ARG,
              "sf_fpfh_block_begin: bad arguments");
-  SF_REQUIRE(radius > 0.0 && radius * 1.0005 <= g->cell, SF_ERR_ARG,
+  SF_REQUIRE(radius_fits(g, radius), SF_ERR_ARG,
              "sf_fpfh_block_begin: radius %g exceeds the cell edge %g the grid was built for", radius, g->cell);
   *total_host = 0;
   if (count == 0) {
     SF_CUDA(cudaMemsetAsync(cand_offsets, 0, 8, stream));
     return SF_OK;
   }
-  int64_t* cand = nullptr;
-  void* scan_temp = nullptr;
-  size_t scan_bytes = 0;
-  cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, cand, cand_offsets, int(count + 1), stream);
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&cand), size_t(count + 1) * 8, stream));
-  SF_CUDA(scratch_alloc(&scan_temp, scan_bytes + 16, stream));
-  SF_CUDA(cudaMemsetAsync(cand + count, 0, 8, stream));
-  self_candidate_count_kernel<<<unsigned((count + 255) / 256), 256, 0, stream>>>(g->view(), first, count, cand);
-  SF_CUDA(cub::DeviceScan::ExclusiveSum(scan_temp, scan_bytes, cand, cand_offsets, int(count + 1), stream));
-  SF_CUDA(cudaMemcpyAsync(total_host, cand_offsets + count, 8, cudaMemcpyDeviceToHost, stream));
-  SF_CUDA(cudaStreamSynchronize(stream));
-  cudaFreeAsync(cand, stream);
-  cudaFreeAsync(scan_temp, stream);
-  return SF_OK;
+  Scratch scratch(stream);
+  return fpfh_candidates(g, first, count, cand_offsets, total_host, scratch, stream);
 }
 
 extern "C" int sf_fpfh_block_spfh(sf_grid* g, double radius, int32_t n_bins, int32_t decorrelated,
@@ -747,29 +748,18 @@ extern "C" int sf_fpfh_block_spfh(sf_grid* g, double radius, int32_t n_bins, int
   if (pairs_host) *pairs_host = 0;
   if (count == 0) return SF_OK;
   SF_REQUIRE(cand_offsets && nbr && weights && counts && spfh_block, SF_ERR_ARG, "sf_fpfh_block_spfh: null argument");
-  SF_REQUIRE(n_bins >= 1 && n_bins <= kMaxBins, SF_ERR_CAPACITY, "sf_fpfh_block_spfh: n_bins must be in [1, %d]", kMaxBins);
-  const int64_t width64 = decorrelated ? 3 * int64_t(n_bins) : int64_t(n_bins) * n_bins * n_bins;
-  SF_REQUIRE(width64 <= 8192, SF_ERR_CAPACITY, "sf_fpfh_block_spfh: histogram width %lld exceeds 8192", (long long)width64);
-  int stride = 0, rows4 = 0;
-  fpfh_row_layout(int(width64), &stride, &rows4);
+  int width = 0, stride = 0, rows4 = 0;
+  if (int rc = histogram_width("sf_fpfh_block_spfh", n_bins, decorrelated, &width)) return rc;
+  fpfh_row_layout(width, &stride, &rows4);
+  Scratch scratch(stream);
   unsigned long long* pair_counter = nullptr;
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&pair_counter), 8, stream));
+  SF_CUDA(scratch.alloc(&pair_counter, 8));
   SF_CUDA(cudaMemsetAsync(pair_counter, 0, 8, stream));
-  const size_t smem = size_t(kSearchWarps) * sizeof(SearchStage);
-  SF_CUDA(cudaFuncSetAttribute(search_weights_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  const int64_t tiles = (count + 31) / 32;
-  search_weights_kernel<<<unsigned((tiles + kSearchWarps - 1) / kSearchWarps), kSearchWarps * 32, smem, stream>>>(
-      g->view(), first, count, radius * radius, cand_offsets, nbr, weights, counts, pair_counter);
-  SF_CUDA(cudaGetLastError());
-  int rc = launch_spfh(g, first, count, cand_offsets, counts, nbr, n_bins, decorrelated, edges_host, spfh_block, stride, stream);
-  if (rc == SF_OK && pairs_host != nullptr) {
-    unsigned long long pairs = 0;
-    SF_CUDA(cudaMemcpyAsync(&pairs, pair_counter, 8, cudaMemcpyDeviceToHost, stream));
-    SF_CUDA(cudaStreamSynchronize(stream));
-    *pairs_host = int64_t(pairs);
-  }
-  cudaFreeAsync(pair_counter, stream);
-  return rc;
+  if (int rc = fpfh_search(g, radius, first, count, cand_offsets, nbr, weights, counts, pair_counter, stream)) return rc;
+  if (int rc = launch_spfh(g, first, count, cand_offsets, counts, nbr, n_bins, decorrelated, edges_host, spfh_block,
+                           stride, stream))
+    return rc;
+  return pairs_host != nullptr ? read_pairs(pair_counter, pairs_host, stream) : SF_OK;
 }
 
 extern "C" int sf_fpfh_block_rows(sf_grid* g, int64_t first, int64_t count, const int64_t* cand_offsets,

@@ -521,7 +521,7 @@ extern "C" int sf_radius_count(sf_grid* g, const double* queries, int64_t self_f
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   SF_REQUIRE(g != nullptr && g->n > 0, SF_ERR_ARG, "sf_radius_count: grid not built");
   SF_REQUIRE(offsets != nullptr && nq >= 0, SF_ERR_ARG, "sf_radius_count: bad arguments");
-  SF_REQUIRE(radius > 0.0 && radius * 1.0005 <= g->cell, SF_ERR_ARG,
+  SF_REQUIRE(radius_fits(g, radius), SF_ERR_ARG,
              "sf_radius_count: radius %g exceeds the cell edge %g the grid was built for", radius, g->cell);
   if (queries == nullptr)
     SF_REQUIRE(self_first >= 0 && self_first + nq <= g->n, SF_ERR_ARG, "self-query range [%lld, %lld) outside the cloud",
@@ -561,7 +561,7 @@ extern "C" int sf_radius_fill(sf_grid* g, const double* queries, int64_t self_fi
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   SF_REQUIRE(g != nullptr && g->n > 0, SF_ERR_ARG, "sf_radius_fill: grid not built");
   SF_REQUIRE(offsets != nullptr && nq >= 0, SF_ERR_ARG, "sf_radius_fill: bad arguments");
-  SF_REQUIRE(radius > 0.0 && radius * 1.0005 <= g->cell, SF_ERR_ARG, "sf_radius_fill: radius exceeds the cell edge");
+  SF_REQUIRE(radius_fits(g, radius), SF_ERR_ARG, "sf_radius_fill: radius exceeds the cell edge");
   if (queries == nullptr)
     SF_REQUIRE(self_first >= 0 && self_first + nq <= g->n, SF_ERR_ARG, "self-query range [%lld, %lld) outside the cloud",
                (long long)self_first, (long long)(self_first + nq));

@@ -113,10 +113,6 @@ __global__ void __launch_bounds__(256)
   }
 }
 
-static bool radius_fits(const sf_grid* g, double radius) {
-  return radius > 0.0 && std::isfinite(radius) && radius * 1.0005 <= g->cell;
-}
-
 }  // namespace sf
 
 using namespace sf;
@@ -161,44 +157,29 @@ extern "C" int sf_iss_select(sf_grid* g, const double* saliency, double non_max_
   auto up = [](size_t b) { return (b + 255) / 256 * 256; };
   const size_t cand_bytes = up(size_t(n) * sizeof(int32_t)), flag_bytes = up(size_t(n)), num_bytes = 256;
   const size_t temp_bytes = up(std::max(if_bytes, flagged_bytes));
-  void* scratch = nullptr;
-  SF_CUDA(scratch_alloc(&scratch, cand_bytes + flag_bytes + num_bytes + temp_bytes, stream));
-  char* base = static_cast<char*>(scratch);
+  Scratch scratch(stream);
+  char* base = nullptr;
+  SF_CUDA(scratch.alloc(&base, cand_bytes + flag_bytes + num_bytes + temp_bytes));
   int32_t* cand = reinterpret_cast<int32_t*>(base);
   uint8_t* flags = reinterpret_cast<uint8_t*>(base + cand_bytes);
   int32_t* nums = reinterpret_cast<int32_t*>(base + cand_bytes + flag_bytes);  // [0] candidates, [1] keypoints
   void* temp = base + cand_bytes + flag_bytes + num_bytes;
-  int rc = SF_OK;
+  size_t bytes = temp_bytes;
+  SF_CUDA(cub::DeviceSelect::If(temp, bytes, positions, cand, nums, n, PositiveSaliency{saliency}, stream));
+  SF_CUDA(cudaMemsetAsync(flags, 0, size_t(n), stream));
+  int blocks = 0, device = 0;
+  cudaGetDevice(&device);
+  cudaDeviceGetAttribute(&blocks, cudaDevAttrMultiProcessorCount, device);
+  // enough warps to cover the SMs several times over; each walks the candidates with a grid stride
+  const int64_t want = std::min<int64_t>(int64_t(blocks) * 8, (int64_t(n) + 7) / 8);
+  iss_nms_kernel<<<unsigned(std::max<int64_t>(want, 1)), 256, 0, stream>>>(
+      g->view(), saliency, cand, nums, non_max_radius * non_max_radius, min_neighbors, flags);
+  SF_CUDA(cudaGetLastError());
+  bytes = temp_bytes;
+  SF_CUDA(cub::DeviceSelect::Flagged(temp, bytes, positions, flags, keypoints, nums + 1, n, stream));
   int32_t selected = 0;
-  do {
-    size_t bytes = temp_bytes;
-    cudaError_t err = cub::DeviceSelect::If(temp, bytes, positions, cand, nums, n, PositiveSaliency{saliency}, stream);
-    if (err == cudaSuccess) err = cudaMemsetAsync(flags, 0, size_t(n), stream);
-    if (err == cudaSuccess) {
-      int blocks = 0, device = 0;
-      cudaGetDevice(&device);
-      cudaDeviceGetAttribute(&blocks, cudaDevAttrMultiProcessorCount, device);
-      // enough warps to cover the SMs several times over; each walks the candidates with a grid stride
-      const int64_t want = std::min<int64_t>(int64_t(blocks) * 8, (int64_t(n) + 7) / 8);
-      iss_nms_kernel<<<unsigned(std::max<int64_t>(want, 1)), 256, 0, stream>>>(
-          g->view(), saliency, cand, nums, non_max_radius * non_max_radius, min_neighbors, flags);
-      err = cudaGetLastError();
-    }
-    if (err == cudaSuccess) {
-      bytes = temp_bytes;
-      err = cub::DeviceSelect::Flagged(temp, bytes, positions, flags, keypoints, nums + 1, n, stream);
-    }
-    if (err == cudaSuccess) err = cudaMemcpyAsync(&selected, nums + 1, sizeof(int32_t), cudaMemcpyDeviceToHost, stream);
-    if (err != cudaSuccess) {
-      sf::set_error("sf_iss_select: %s", cudaGetErrorString(err));
-      rc = SF_ERR_CUDA;
-    }
-  } while (false);
-  const cudaError_t freed = cudaFreeAsync(scratch, stream);
-  const cudaError_t synced = cudaStreamSynchronize(stream);
-  if (rc != SF_OK) return rc;
-  SF_CUDA(freed);
-  SF_CUDA(synced);
+  SF_CUDA(cudaMemcpyAsync(&selected, nums + 1, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+  SF_CUDA(cudaStreamSynchronize(stream));
   *count_host = selected;
   return SF_OK;
 }

@@ -464,9 +464,10 @@ extern "C" int sf_nonempty_rows(const double* desc, int64_t n, int32_t width, in
   size_t temp_bytes = 0;
   cub::CountingInputIterator<int64_t> ids(0);
   cub::DeviceSelect::Flagged(nullptr, temp_bytes, ids, flags, rows, count_dev, int(n), stream);
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&flags), size_t(n), stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&count_dev), 2 * sizeof(int64_t), stream));
-  SF_CUDA(scratch_alloc(&temp, temp_bytes + 16, stream));
+  Scratch scratch(stream);
+  SF_CUDA(scratch.alloc(&flags, size_t(n)));
+  SF_CUDA(scratch.alloc(&count_dev, 2 * sizeof(int64_t)));
+  SF_CUDA(scratch.alloc(&temp, temp_bytes + 16));
   unsigned long long* absmax_dev = reinterpret_cast<unsigned long long*>(count_dev + 1);
   SF_CUDA(cudaMemsetAsync(absmax_dev, 0, sizeof(unsigned long long), stream));
   nonempty_kernel<<<unsigned((n * 32 + 255) / 256), 256, 0, stream>>>(desc, n, width, flags,
@@ -474,9 +475,6 @@ extern "C" int sf_nonempty_rows(const double* desc, int64_t n, int32_t width, in
   SF_CUDA(cub::DeviceSelect::Flagged(temp, temp_bytes, ids, flags, rows, count_dev, int(n), stream));
   SF_CUDA(cudaMemcpyAsync(count_host, count_dev, sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
   if (absmax_host) SF_CUDA(cudaMemcpyAsync(absmax_host, absmax_dev, sizeof(double), cudaMemcpyDeviceToHost, stream));
-  SF_CUDA(cudaFreeAsync(flags, stream));
-  SF_CUDA(cudaFreeAsync(count_dev, stream));
-  SF_CUDA(cudaFreeAsync(temp, stream));
   SF_CUDA(cudaStreamSynchronize(stream));
   return SF_OK;
 }
@@ -634,23 +632,21 @@ extern "C" int sf_match_exhaustive(const double* a, const int64_t* rows_a, const
              "sf_match_exhaustive: scale and norm_bound must be finite");
   SF_REQUIRE(qb < (int64_t(1) << 31), SF_ERR_ARG, "sf_match_exhaustive: too many targets");
   if (n_which == 0) return SF_OK;
+  const int64_t query_tiles = (n_which + kEx32Rows - 1) / kEx32Rows;
+  SF_REQUIRE(query_tiles <= 65535, SF_ERR_CAPACITY, "sf_match_exhaustive: %lld flagged queries", (long long)n_which);
   int32_t* counts = nullptr;
   double* list_d = nullptr;
   int32_t* list_i = nullptr;
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&counts), size_t(n_which) * 4, stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&list_d), size_t(n_which) * kExhaustiveCap * 8, stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&list_i), size_t(n_which) * kExhaustiveCap * 4, stream));
+  Scratch scratch(stream);
+  SF_CUDA(scratch.alloc(&counts, size_t(n_which) * 4));
+  SF_CUDA(scratch.alloc(&list_d, size_t(n_which) * kExhaustiveCap * 8));
+  SF_CUDA(scratch.alloc(&list_i, size_t(n_which) * kExhaustiveCap * 4));
   SF_CUDA(cudaMemsetAsync(counts, 0, size_t(n_which) * 4, stream));
-  const int64_t query_tiles = (n_which + kEx32Rows - 1) / kEx32Rows;
-  SF_REQUIRE(query_tiles <= 65535, SF_ERR_CAPACITY, "sf_match_exhaustive: %lld flagged queries", (long long)n_which);
   const dim3 grid(unsigned((qb + kEx32Rows - 1) / kEx32Rows), unsigned(query_tiles));
   exhaustive_tile32_kernel<<<grid, 256, 0, stream>>>(a, rows_a, which, n_which, limit, b, rows_b, qb, width, scale, norm_bound,
                                                      counts, list_d, list_i);
   exhaustive_select_kernel<<<unsigned((n_which + 127) / 128), 128, 0, stream>>>(n_which, counts, list_d, list_i, cand16);
   SF_CUDA(cudaGetLastError());
-  cudaFreeAsync(counts, stream);
-  cudaFreeAsync(list_d, stream);
-  cudaFreeAsync(list_i, stream);
   return SF_OK;
 }
 

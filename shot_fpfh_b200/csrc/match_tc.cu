@@ -434,8 +434,9 @@ int launch_topk_tc(const __half* a, int64_t qa, const __half* b, const float* bn
   const int parts = kEpiParts * splits;
   float* part_score = nullptr;
   int32_t* part_idx = nullptr;
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&part_score), size_t(parts) * qa * k * sizeof(float), stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&part_idx), size_t(parts) * qa * k * sizeof(int32_t), stream));
+  Scratch scratch(stream);
+  SF_CUDA(scratch.alloc(&part_score, size_t(parts) * qa * k * sizeof(float)));
+  SF_CUDA(scratch.alloc(&part_idx, size_t(parts) * qa * k * sizeof(int32_t)));
   const int num_kb = wp / kBK;
   int rc = SF_OK;
   switch (k) {
@@ -445,10 +446,8 @@ int launch_topk_tc(const __half* a, int64_t qa, const __half* b, const float* bn
     case 8: rc = launch<8>(map_a, map_b, bnorm, qa, qb, num_kb, splits, tiles_per_split, index_offset, part_score, part_idx, stream); break;
     default: rc = launch<16>(map_a, map_b, bnorm, qa, qb, num_kb, splits, tiles_per_split, index_offset, part_score, part_idx, stream); break;
   }
-  if (rc == SF_OK) rc = launch_merge_partials(part_score, part_idx, parts, qa, k, score, idx, stream);
-  cudaFreeAsync(part_score, stream);
-  cudaFreeAsync(part_idx, stream);
-  return rc;
+  if (rc != SF_OK) return rc;
+  return launch_merge_partials(part_score, part_idx, parts, qa, k, score, idx, stream);
 }
 
 }  // namespace sf

@@ -142,7 +142,7 @@ extern "C" int sf_knn(sf_grid* g, const double* queries, int64_t nq, int32_t k, 
   SF_REQUIRE(g != nullptr && g->n > 0, SF_ERR_ARG, "sf_knn: grid not built");
   SF_REQUIRE(queries && nbr_index && status && nq >= 0, SF_ERR_ARG, "sf_knn: bad arguments");
   SF_REQUIRE(k >= 1 && k <= kKnnCapacity, SF_ERR_CAPACITY, "sf_knn: k must be in [1, %d]", kKnnCapacity);
-  SF_REQUIRE(reach > 0.0 && reach * 1.0005 <= g->cell, SF_ERR_ARG, "sf_knn: reach exceeds the grid's cell edge");
+  SF_REQUIRE(radius_fits(g, reach), SF_ERR_ARG, "sf_knn: reach exceeds the grid's cell edge");
   if (nq == 0) return SF_OK;
   knn_kernel<<<unsigned((nq + 3) / 4), 128, 0, stream>>>(g->view(), queries, nq, k, reach * reach, nbr_index, status);
   SF_CUDA(cudaGetLastError());

@@ -148,24 +148,22 @@ extern "C" int sf_icp_plane_step(sf_grid* g, const double* scan, int64_t n_scan,
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   SF_REQUIRE(g != nullptr && g->n > 0 && g->has_normals, SF_ERR_ARG, "sf_icp_plane_step: grid built without normals");
   SF_REQUIRE(scan && transform_host && sums_host && n_scan >= 0, SF_ERR_ARG, "sf_icp_plane_step: null argument");
-  SF_REQUIRE(d_max > 0.0 && d_max * 1.0005 <= g->cell, SF_ERR_ARG,
+  SF_REQUIRE(radius_fits(g, d_max), SF_ERR_ARG,
              "sf_icp_plane_step: d_max %g exceeds the cell edge %g the grid was built for", d_max, g->cell);
   for (int k = 0; k < kIcpTerms; ++k) sums_host[k] = 0.0;
   if (n_scan == 0) return SF_OK;
   const int64_t blocks = std::min<int64_t>((n_scan * 32 + 255) / 256, 148 * 8);
   const int64_t warps = blocks * 8;
   double *transform = nullptr, *partial = nullptr, *sums = nullptr;
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&transform), 12 * sizeof(double), stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&partial), size_t(warps) * kIcpTerms * sizeof(double), stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&sums), kIcpTerms * sizeof(double), stream));
+  Scratch scratch(stream);
+  SF_CUDA(scratch.alloc(&transform, 12 * sizeof(double)));
+  SF_CUDA(scratch.alloc(&partial, size_t(warps) * kIcpTerms * sizeof(double)));
+  SF_CUDA(scratch.alloc(&sums, kIcpTerms * sizeof(double)));
   SF_CUDA(cudaMemcpyAsync(transform, transform_host, 12 * sizeof(double), cudaMemcpyHostToDevice, stream));
   icp_plane_kernel<<<unsigned(blocks), 256, 0, stream>>>(g->view(), scan, n_scan, transform, d_max, partial, nearest);
   icp_reduce_kernel<<<1, 32, 0, stream>>>(partial, warps, sums);
   SF_CUDA(cudaGetLastError());
   SF_CUDA(cudaMemcpyAsync(sums_host, sums, kIcpTerms * sizeof(double), cudaMemcpyDeviceToHost, stream));
   SF_CUDA(cudaStreamSynchronize(stream));
-  cudaFreeAsync(transform, stream);
-  cudaFreeAsync(partial, stream);
-  cudaFreeAsync(sums, stream);
   return SF_OK;
 }

@@ -4,6 +4,8 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <cmath>
+
 #include "../../include/shotfpfh_b200.h"
 #include "sf_math.cuh"
 
@@ -34,22 +36,48 @@ void profile_mark(int i, cudaStream_t stream);
     }                                    \
   } while (0)
 
-// Stream-ordered scratch memory. The default memory pool returns freed memory to the OS at every synchronisation
-// (release threshold 0), which made each call re-pay a cudaMalloc (measured: 21 ms per matching step for 0.4 ms of
-// kernels); the threshold is raised once so that the pool keeps what it has been given.
-inline cudaError_t scratch_alloc(void** p, size_t bytes, cudaStream_t stream) {
-  static bool configured = false;
-  if (!configured) {
+// Stream-ordered scratch memory of one call: every buffer alloc() hands out is freed on the stream when the Scratch
+// goes out of scope, whichever way the call returns. The status of the free is ignored: an error that matters surfaces
+// at the call's synchronisation or at the next call.
+class Scratch {
+ public:
+  explicit Scratch(cudaStream_t stream) : stream_(stream) {}
+  Scratch(const Scratch&) = delete;
+  Scratch& operator=(const Scratch&) = delete;
+  ~Scratch() {
+    for (int i = 0; i < count_; ++i) cudaFreeAsync(ptrs_[i], stream_);
+  }
+
+  template <typename T>
+  cudaError_t alloc(T** p, size_t bytes) {
+    if (count_ == kMaxBuffers) return cudaErrorMemoryAllocation;  // more buffers than one call is written for
+    keep_freed_memory();
+    const cudaError_t err = cudaMallocAsync(p, bytes, stream_);
+    if (err == cudaSuccess) ptrs_[count_++] = *p;
+    return err;
+  }
+
+ private:
+  // The default memory pool returns freed memory to the OS at every synchronisation (release threshold 0), which made
+  // each call re-pay a cudaMalloc (measured: 21 ms per matching step for 0.4 ms of kernels); the threshold is raised
+  // once so that the pool keeps what it has been given.
+  static void keep_freed_memory() {
+    static bool configured = false;
+    if (configured) return;
+    configured = true;
     int device = 0;
     cudaMemPool_t pool;
     if (cudaGetDevice(&device) == cudaSuccess && cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess) {
       uint64_t keep = ~uint64_t(0);
       cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
     }
-    configured = true;
   }
-  return cudaMallocAsync(p, bytes, stream);
-}
+
+  static constexpr int kMaxBuffers = 16;
+  cudaStream_t stream_;
+  void* ptrs_[kMaxBuffers];
+  int count_ = 0;
+};
 
 // Device-side view of a built grid (passed by value to kernels).
 struct GridView {
@@ -135,6 +163,12 @@ struct sf_grid {
 };
 
 namespace sf {
+
+// A fixed-radius search on the grid looks at the 27 cells around a query: the radius must not exceed the cell edge
+// (with margin for the rounding of the cell coordinates).
+inline bool radius_fits(const sf_grid* g, double radius) {
+  return radius > 0.0 && std::isfinite(radius) && radius * 1.0005 <= g->cell;
+}
 
 // ---- warp helpers -----------------------------------------------------------------------------------------
 __device__ __forceinline__ double warp_sum(double v) {

@@ -1234,11 +1234,10 @@ extern "C" int sf_shot_descriptor(sf_grid* g, const double* queries, int64_t nq,
   if (nq == 0) return SF_OK;  // (an empty query block has null pointers: zero-row tensors)
   SF_REQUIRE(queries && offsets && lrf && out && nq > 0, SF_ERR_ARG, "sf_shot_descriptor: bad arguments");
   int32_t* worklist = nullptr;
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&worklist), size_t(nq + 1) * 4, stream));
-  const int rc = launch_descriptor(g, queries, nq, radius, offsets, nullptr, nbr, false, const_cast<double*>(lrf), nullptr, 0,
-                                   min_nb, normalize, out, out_is_f64, worklist + 1, worklist, nullptr, stream);
-  cudaFreeAsync(worklist, stream);
-  return rc;
+  Scratch scratch(stream);
+  SF_CUDA(scratch.alloc(&worklist, size_t(nq + 1) * 4));
+  return launch_descriptor(g, queries, nq, radius, offsets, nullptr, nbr, false, const_cast<double*>(lrf), nullptr, 0,
+                           min_nb, normalize, out, out_is_f64, worklist + 1, worklist, nullptr, stream);
 }
 
 // Scratch of the fused driver, kept by the grid handle between calls (the stream-ordered pool cost a dozen
@@ -1281,7 +1280,7 @@ extern "C" int sf_shot_single_scale(sf_grid* g, const double* queries, int64_t n
   if (pairs_host) *pairs_host = 0;
   if (nq == 0) return SF_OK;  // (an empty query block has null pointers: zero-row tensors)
   SF_REQUIRE(queries && out && nq > 0, SF_ERR_ARG, "sf_shot_single_scale: bad arguments");
-  SF_REQUIRE(radius > 0.0 && radius * 1.0005 <= g->cell, SF_ERR_ARG,
+  SF_REQUIRE(radius_fits(g, radius), SF_ERR_ARG,
              "sf_shot_single_scale: radius %g exceeds the cell edge %g the grid was built for", radius, g->cell);
   if (int rc = shot_reserve_queries(g, nq)) return rc;
   int64_t* cand_offsets = g->shot_cand_offsets;

@@ -133,15 +133,16 @@ extern "C" int sf_voxel_subsample(const double* xyz, int64_t n, double voxel, in
   cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, keys_in, keys_out, vals_in, order, int(n), 0, 63, stream);
   cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, flags, rank, int(n), stream);
   const size_t temp_bytes = (sort_bytes > scan_bytes ? sort_bytes : scan_bytes) + 256;
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&lo), 4 * sizeof(unsigned long long), stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&keys_in), size_t(n) * 8, stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&keys_out), size_t(n) * 8, stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&vals_in), size_t(n) * 4, stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&order), size_t(n) * 4, stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&flags), size_t(n) * 4, stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&rank), size_t(n + 1) * 4, stream));
-  SF_CUDA(scratch_alloc(reinterpret_cast<void**>(&overflow), sizeof(int), stream));
-  SF_CUDA(scratch_alloc(&temp, temp_bytes, stream));
+  Scratch scratch(stream);
+  SF_CUDA(scratch.alloc(&lo, 4 * sizeof(unsigned long long)));
+  SF_CUDA(scratch.alloc(&keys_in, size_t(n) * 8));
+  SF_CUDA(scratch.alloc(&keys_out, size_t(n) * 8));
+  SF_CUDA(scratch.alloc(&vals_in, size_t(n) * 4));
+  SF_CUDA(scratch.alloc(&order, size_t(n) * 4));
+  SF_CUDA(scratch.alloc(&flags, size_t(n) * 4));
+  SF_CUDA(scratch.alloc(&rank, size_t(n + 1) * 4));
+  SF_CUDA(scratch.alloc(&overflow, sizeof(int)));
+  SF_CUDA(scratch.alloc(&temp, temp_bytes));
   SF_CUDA(cudaMemsetAsync(overflow, 0, sizeof(int), stream));
   const unsigned blocks = unsigned((n + 255) / 256);
   voxel_min_init_kernel<<<1, 32, 0, stream>>>(lo);
@@ -158,8 +159,6 @@ extern "C" int sf_voxel_subsample(const double* xyz, int64_t n, double voxel, in
   SF_CUDA(cudaMemcpyAsync(&last_rank, rank + (n - 1), sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
   SF_CUDA(cudaMemcpyAsync(&last_flag, flags + (n - 1), sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
   SF_CUDA(cudaMemcpyAsync(&overflow_host, overflow, sizeof(int), cudaMemcpyDeviceToHost, stream));
-  void* to_free[] = {lo, keys_in, keys_out, vals_in, order, flags, rank, overflow, temp};
-  for (void* p : to_free) SF_CUDA(cudaFreeAsync(p, stream));
   SF_CUDA(cudaStreamSynchronize(stream));
   SF_REQUIRE(overflow_host == 0, SF_ERR_CAPACITY, "sf_voxel_subsample: more than 2^21 voxels along an axis");
   *count_host = int64_t(last_rank) + last_flag;

@@ -59,10 +59,10 @@ extern "C" int sf_rows_compact_count(const float* dense, int64_t n_rows, int32_t
   void* temp = nullptr;
   size_t temp_bytes = 0;
   cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, offsets_dev, offsets_dev, int(n_rows + 1), stream);
-  SF_CUDA(scratch_alloc(&temp, temp_bytes + 16, stream));
+  Scratch scratch(stream);
+  SF_CUDA(scratch.alloc(&temp, temp_bytes + 16));
   SF_CUDA(cub::DeviceScan::ExclusiveSum(temp, temp_bytes, offsets_dev, offsets_dev, int(n_rows + 1), stream));
   SF_CUDA(cudaMemcpyAsync(total_host, offsets_dev + n_rows, sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
-  SF_CUDA(cudaFreeAsync(temp, stream));
   SF_CUDA(cudaStreamSynchronize(stream));
   return SF_OK;
 }

@@ -81,6 +81,18 @@ def test_product_never_imports_the_oracle():
                 assert "/root/reference" not in text, os.path.join(dirpath, name)
 
 
+def test_per_call_scratch_has_one_owner():
+    """Per-call device scratch is taken through sf::Scratch (csrc/sf_common.cuh), which frees it on every return path:
+    no other source allocates from or frees to the stream-ordered pool itself."""
+    csrc = os.path.join(ROOT, "shot_fpfh_b200", "csrc")
+    for name in sorted(os.listdir(csrc)):
+        if name.endswith((".cu", ".cuh", ".cpp", ".h")) and name != "sf_common.cuh":
+            with open(os.path.join(csrc, name)) as f:
+                text = f.read()
+            for word in ("cudaMallocAsync", "cudaFreeAsync", "scratch_alloc"):
+                assert word not in text, f"{name} names {word}"
+
+
 def test_signatures_pinned():
     """The reference-shaped API keeps the parameter lists stored in tests/golden/api_signatures.json (what the live
     comparison below checks against the reference itself)."""
