@@ -49,6 +49,13 @@ SF_HD double rdist3(double dx, double dy, double dz) {
   return add_rn(add_rn(mul_rn(dx, dx), mul_rn(dy, dy)), mul_rn(dz, dz));
 }
 
+// One coordinate in the local frame, c . (column of the frame), rounded as the oracle's `rel @ lrf` rounds it: NumPy's
+// float64 matmul (OpenBLAS dgemm) accumulates k = 0, 1, 2 with fused multiply-adds. On a plane Z is rounding noise of
+// either sign and its sign picks the elevation bin, so the order of the roundings is part of the result there.
+SF_HD double frame_dot(double cx, double cy, double cz, double f0, double f1, double f2) {
+  return fma(cz, f2, fma(cy, f1, mul_rn(cx, f0)));
+}
+
 // ----------------------------------------------------------------------------------------------------------
 // SHOT: one neighbour -> its own bin, the five "other" targets and the six values (SURVEY.md Appendix A).
 // ----------------------------------------------------------------------------------------------------------
@@ -98,11 +105,18 @@ struct ShotDecision {
   int own, cos_nb, az_nb;  // flat bins: own, statement-1 target, statement-9 target
   uint32_t key;            // distance order (see ShotRecord::key)
   int ti, ei, saz;         // azimuth octant, elevation bit, sign of the azimuth offset from the octant centre
+  bool equator;            // Z > 0 but the reference's float64 phi = arccos(Z / rho) is exactly pi / 2 (see below)
   float a_cos;             // |cosine offset| (statement 1 value; 1 - a_cos goes to the own bin)
   float own_shell;         // radial weight of the own bin (statement 5)
   float other_shell;       // radial weight sent to the OTHER shell (statement 3 or 4)
   float fx, fy, ratio;     // float32 inputs of the two transcendental weights: atan2f(fy, fx), acosf(ratio)
 };
+
+// Largest Z / rho > 0 whose float64 arccos is exactly pi / 2 (np.arccos, glibc's correctly rounded acos): the double
+// pi / 2 lies 6.1e-17 below the true value, so arccos(t) = pi/2 - t rounds to it up to t = half an ulp + 6.1e-17.
+// On a plane that is not axis-aligned, Z of an in-plane neighbour is rounding noise of either sign (|Z| ~ 1e-17 rho),
+// so about half of the neighbours land in this window. tests/test_host_math.py pins the value against np.arccos.
+constexpr double kAcosHalfPiMax = 1.7225464241988333e-16;
 
 SF_HD ShotDecision shot_decide(double X, double Y, double Z, double cosine, double rho, double radius, double inv_radius) {
   ShotDecision d;
@@ -113,6 +127,9 @@ SF_HD ShotDecision shot_decide(double X, double Y, double Z, double cosine, doub
   const int scos = (dcos > 0.0) - (dcos < 0.0);
   d.ti = azimuth_octant(X, Y);
   d.ei = Z > 0.0;
+  // the reference bins by Z > 0 but interpolates by phi: with phi == pi/2 its statement 7 (`lower`, phi < pi/2)
+  // writes 0 although the neighbour sits in the upper half (the division only runs for |Z| below 1e-15 rho)
+  d.equator = Z > 0.0 && Z < 1e-15 * rho && Z / rho <= kAcosHalfPiMax;
   const int ri = rho > radius / 2;
   d.own = shot_flat(ci, d.ti, d.ei, ri);
   int cnb = ci + scos;
@@ -145,13 +162,13 @@ SF_HD ShotDecision shot_decide(double X, double Y, double Z, double cosine, doub
 }
 
 // ---- step 2: the two transcendental weights, float32 (continuous in their inputs) ---------------------------------
-// elevation (shot.py:142-171): phi < pi/2 <=> Z > 0 (see DESIGN.md)
+// elevation (shot.py:142-171): phi < pi/2 <=> Z > 0 (see DESIGN.md), except in the window of kAcosHalfPiMax
 SF_HD void shot_elevation(const ShotDecision& d, float& own_vol, float& other_vol) {
   const float kPi = 3.14159265358979323846f, inv_h = 0.63661977236758134308f;  // 1 / (pi / 2)
   const float phi = acosf(d.ratio);
   if (d.ei) {  // upper half-space, elevation bin 1, centre pi/4; statement 7 carries `lower`
     own_vol = 1.0f - fabsf(phi - 0.25f * kPi) * inv_h;
-    other_vol = phi >= 0.25f * kPi ? (phi - 0.25f * kPi) * inv_h : 0.0f;
+    other_vol = phi >= 0.25f * kPi && !d.equator ? (phi - 0.25f * kPi) * inv_h : 0.0f;
   } else {     // Z <= 0, elevation bin 0, centre 3pi/4; statement 6 carries `upper`
     own_vol = 1.0f - fabsf(phi - 0.75f * kPi) * inv_h;
     other_vol = phi <= 0.75f * kPi ? (0.75f * kPi - phi) * inv_h : 0.0f;
@@ -278,6 +295,7 @@ SF_HD bool shot_decide_fast(float X, float Y, float Z, float cosine, float rho, 
   const bool second = (upper == right) ? !wide : wide;  // azimuth_octant with X, Y != 0
   d.ti = 4 * int(upper) + 2 * int(right != upper) + int(second);
   d.ei = Z > 0.0f;
+  d.equator = false;  // a sure decision has |Z| > e_loc >= 8 u rho, far above the window of kAcosHalfPiMax
   const float half = 0.5f * radius;
   const int ri = rho > half;
   sure = sure && fabsf(rho - half) > m.e_rho && rho < radius * 1.001f && rho > m.w_rho_min && hi > m.w_xy_min;
@@ -392,17 +410,25 @@ SF_HD bool shot_keys_ambiguous(uint32_t a, uint32_t b, uint32_t margin) {
 // neighbour of own bin b addresses the same radial partner b^1 (and elevation partner b^2): the winner of the slot
 // "radial statement, bins {b, b^1}" is whichever of the two own-bin winners is farther, and it contributes its
 // `other_shell` weight to the bin it is NOT in (0 to its own). So per query:
-//   keys  uint32 [3][352] : distance key of the winner of {own-bin group, statement 1, statement 9}, 0 = nobody
+//   keys  uint64 [3][352] : order key (shot_order_key) of the winner of {own-bin group, statement 1, statement 9},
+//                           0 = nobody
 //   vals  float  [5][352] : v_own, v_rad (other_shell), v_el (other_vol) of the own-bin winner; v_cos; v_az
-// Keys are raised with a native 32-bit atomicMax; after a warp barrier the lanes whose key is (still) the slot's key
-// store their values. Two DIFFERENT neighbours with the same 32-bit key on one slot (distances within
-// radius * 2^-32) are an exact-distance tie: one of them wins, as in the reference's unstable argsort.
+// Keys are raised with a native 64-bit atomicMax; after a barrier the lane whose key is (still) the slot's key stores
+// its values. The key is the 32-bit distance key, then the neighbour's position in the query's list: keys are unique
+// inside a query, so two neighbours at the same distance (exact ties, or distances within radius * 2^-32) cannot both
+// win a slot, and the later one in the list wins whatever the schedule — the warp kernel, the block kernel and a
+// repeated call give the same row. (The reference breaks such ties by its unstable argsort: the tie itself stays an
+// exemption, DESIGN.md §2.)
+SF_HD uint64_t shot_order_key(uint32_t distance_key, uint32_t position) {
+  return (uint64_t(distance_key) << 32) | position;
+}
 constexpr int kKeyOwn = 0, kKeyCos = kShotLen, kKeyAz = 2 * kShotLen, kKeyCount = 3 * kShotLen;
 constexpr int kValOwn = 0, kValRad = kShotLen, kValEl = 2 * kShotLen, kValCos = 3 * kShotLen, kValAz = 4 * kShotLen,
               kValCount = 5 * kShotLen;
 
-SF_HD float shot_bin_value_compact(const uint32_t* keys, const float* vals, int flat) {
-  const uint32_t k_own = keys[kKeyOwn + flat];
+template <typename Key>
+SF_HD float shot_bin_value_compact(const Key* keys, const float* vals, int flat) {
+  const Key k_own = keys[kKeyOwn + flat];
   float v = k_own ? vals[kValOwn + flat] : 0.0f;
   if (keys[kKeyCos + flat]) v += vals[kValCos + flat];
   if (keys[kKeyAz + flat]) v += vals[kValAz + flat];
@@ -415,7 +441,8 @@ SF_HD float shot_bin_value_compact(const uint32_t* keys, const float* vals, int 
 
 // The same assembly for the four bins {4g .. 4g+3} of one (cosine, azimuth) cell at once: their radial / elevation
 // partners are inside the group, so a lane needs exactly eight 16-byte table reads (what the kernel does).
-SF_HD void shot_bin_group_compact(const uint32_t ko[4], const uint32_t kc[4], const uint32_t ka[4], const float vo[4],
+template <typename Key>
+SF_HD void shot_bin_group_compact(const Key ko[4], const Key kc[4], const Key ka[4], const float vo[4],
                                   const float vr[4], const float ve[4], const float vc[4], const float va[4],
                                   float out[4]) {
 #if defined(__CUDA_ARCH__)

@@ -5,7 +5,7 @@
 // S2 implements the reference's actual semantics (SURVEY.md F1 / Appendix A): its ten `descriptor[idx] += v`
 // statements are buffered NumPy fancy-index updates, so per statement and per bin only the neighbour with the
 // largest distance that addresses the bin contributes (even with value 0). Each warp owns compact winner tables in
-// shared memory (sf_math.cuh: three uint32 key tables raised with the native 32-bit atomicMax, five float value
+// shared memory (sf_math.cuh: three uint64 key tables raised with the native 64-bit atomicMax, five float value
 // tables written by the lanes that still hold a slot's key after a warp barrier); bins then sum their statements.
 #include <cub/cub.cuh>
 
@@ -331,12 +331,18 @@ __global__ void __launch_bounds__(256)
 }
 
 // ---- S2 ----------------------------------------------------------------------------------------------------
-// Per warp: uint32 keys[3][352] + float vals[5][352] = 11 264 B of shared memory (sf_math.cuh, "winner tables,
-// compact form"). Per 32 neighbours: (a) float64 decisions, (b) three native 32-bit atomicMax on the key tables,
+// Per warp: uint64 keys[3][352] + float vals[5][352] = 15 488 B of shared memory (sf_math.cuh, "winner tables,
+// compact form"). Per 32 neighbours: (a) float64 decisions, (b) three native 64-bit atomicMax on the key tables,
 // (c) warp barrier, (d) the lanes that hold a slot's key compute the transcendental weights they need (only winners
 // pay for acosf / atan2f) and store their values. After the last neighbour each lane assembles 11 bins.
 constexpr int kShotWarpsPerBlock = 4;
-constexpr int kShotSmemPerWarp = (kKeyCount + kValCount) * 4;
+
+// Four consecutive 64-bit keys (32-byte aligned) as two 16-byte shared-memory reads.
+__device__ __forceinline__ void load_keys4(const unsigned long long* k, unsigned long long out[4]) {
+  const ulonglong2 a = reinterpret_cast<const ulonglong2*>(k)[0], b = reinterpret_cast<const ulonglong2*>(k)[1];
+  out[0] = a.x; out[1] = a.y; out[2] = b.x; out[3] = b.y;
+}
+constexpr int kShotSmemPerWarp = kKeyCount * 8 + kValCount * 4;
 
 // 352 * sizeof(OutT) is a multiple of 16, so every row and every group of four bins is 16-byte aligned
 __device__ __forceinline__ void store_group(float* p, float a, float b, float c, float d) {
@@ -368,7 +374,7 @@ __global__ void __launch_bounds__(kShotWarpsPerBlock * 32, 5)
   extern __shared__ uint32_t table_mem[];
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
-  uint32_t* keys = table_mem + warp * (kKeyCount + kValCount);
+  unsigned long long* keys = reinterpret_cast<unsigned long long*>(table_mem + warp * (kShotSmemPerWarp / 4));
   float* vals = reinterpret_cast<float*>(keys + kKeyCount);
   const int64_t warps_total = int64_t(gridDim.x) * kShotWarpsPerBlock;
   const double inv_radius = 1.0 / radius;
@@ -377,7 +383,7 @@ __global__ void __launch_bounds__(kShotWarpsPerBlock * 32, 5)
   for (int64_t item = blockIdx.x * int64_t(kShotWarpsPerBlock) + warp; item < n_items; item += warps_total) {
     const int64_t q = worklist != nullptr ? int64_t(worklist[item]) : item;
     // values are gated by their keys: only the keys are cleared (16 bytes per lane and store)
-    for (int j = lane; j < kKeyCount / 4; j += 32) reinterpret_cast<uint4*>(keys)[j] = make_uint4(0u, 0u, 0u, 0u);
+    for (int j = lane; j < kKeyCount / 2; j += 32) reinterpret_cast<uint4*>(keys)[j] = make_uint4(0u, 0u, 0u, 0u);
     const double qx = __ldg(queries + 3 * q), qy = __ldg(queries + 3 * q + 1), qz = __ldg(queries + 3 * q + 2);
     const int64_t begin = offsets[q], end = counts ? begin + counts[q] : offsets[q + 1];
     double f[9];
@@ -434,6 +440,7 @@ __global__ void __launch_bounds__(kShotWarpsPerBlock * 32, 5)
         if (i + 64 < end) s_after = __ldg(nbr + (i + 64) * nbr_stride + nbr_word) & 0x7fffffff;
       }
       ShotDecision d;
+      unsigned long long key = 0;
       bool active = false;
       if (i < end) {
         const double cx = p.x - qx, cy = p.y - qy, cz = p.z - qz;
@@ -442,22 +449,23 @@ __global__ void __launch_bounds__(kShotWarpsPerBlock * 32, 5)
           active = true;
           ++positive;
           const double rho = sqrt(d2);
-          const double X = cx * f[0] + cy * f[3] + cz * f[6];
-          const double Y = cx * f[1] + cy * f[4] + cz * f[7];
-          const double Z = cx * f[2] + cy * f[5] + cz * f[8];
+          const double X = frame_dot(cx, cy, cz, f[0], f[3], f[6]);
+          const double Y = frame_dot(cx, cy, cz, f[1], f[4], f[7]);
+          const double Z = frame_dot(cx, cy, cz, f[2], f[5], f[8]);
           double cosine = n.x * f[2] + n.y * f[5] + n.z * f[8];
           cosine = fmin(1.0, fmax(-1.0, cosine));
           d = shot_decide(X, Y, Z, cosine, rho, radius, inv_radius);
-          atomicMax(keys + kKeyOwn + d.own, d.key);
-          atomicMax(keys + kKeyCos + d.cos_nb, d.key);
-          atomicMax(keys + kKeyAz + d.az_nb, d.key);
+          key = shot_order_key(d.key, uint32_t(i - begin));
+          atomicMax(keys + kKeyOwn + d.own, key);
+          atomicMax(keys + kKeyCos + d.cos_nb, key);
+          atomicMax(keys + kKeyAz + d.az_nb, key);
         }
       }
       __syncwarp();
       if (active) {
-        const bool win_own = keys[kKeyOwn + d.own] == d.key;
-        const bool win_cos = keys[kKeyCos + d.cos_nb] == d.key;
-        const bool win_az = keys[kKeyAz + d.az_nb] == d.key;
+        const bool win_own = keys[kKeyOwn + d.own] == key;
+        const bool win_cos = keys[kKeyCos + d.cos_nb] == key;
+        const bool win_az = keys[kKeyAz + d.az_nb] == key;
         float a_az = 0.0f;
         if (win_own || win_az) a_az = shot_azimuth(d);
         if (win_own) {
@@ -483,16 +491,15 @@ __global__ void __launch_bounds__(kShotWarpsPerBlock * 32, 5)
     for (int j = 0; j < kGroupRounds; ++j) {
       const int grp = lane + 32 * j;
       if (grp < kGroups) {
-        const uint4 ko = *reinterpret_cast<const uint4*>(keys + kKeyOwn + 4 * grp);
-        const uint4 kc = *reinterpret_cast<const uint4*>(keys + kKeyCos + 4 * grp);
-        const uint4 ka = *reinterpret_cast<const uint4*>(keys + kKeyAz + 4 * grp);
+        unsigned long long ko_[4], kc_[4], ka_[4];
+        load_keys4(keys + kKeyOwn + 4 * grp, ko_);
+        load_keys4(keys + kKeyCos + 4 * grp, kc_);
+        load_keys4(keys + kKeyAz + 4 * grp, ka_);
         const float4 vo = *reinterpret_cast<const float4*>(vals + kValOwn + 4 * grp);
         const float4 vr = *reinterpret_cast<const float4*>(vals + kValRad + 4 * grp);
         const float4 ve = *reinterpret_cast<const float4*>(vals + kValEl + 4 * grp);
         const float4 vc = *reinterpret_cast<const float4*>(vals + kValCos + 4 * grp);
         const float4 va = *reinterpret_cast<const float4*>(vals + kValAz + 4 * grp);
-        const uint32_t ko_[4] = {ko.x, ko.y, ko.z, ko.w}, kc_[4] = {kc.x, kc.y, kc.z, kc.w},
-                       ka_[4] = {ka.x, ka.y, ka.z, ka.w};
         const float vo_[4] = {vo.x, vo.y, vo.z, vo.w}, vr_[4] = {vr.x, vr.y, vr.z, vr.w},
                     ve_[4] = {ve.x, ve.y, ve.z, ve.w}, vc_[4] = {vc.x, vc.y, vc.z, vc.w},
                     va_[4] = {va.x, va.y, va.z, va.w};
@@ -534,7 +541,7 @@ __global__ void __launch_bounds__(kBlockQueryWarps * 32)
                                  const int32_t* __restrict__ work_count, int nbr_stride,
                                  const int32_t* __restrict__ status) {
   if (status != nullptr && *status != 0) return;
-  __shared__ __align__(16) uint32_t keys[kKeyCount];
+  __shared__ __align__(16) unsigned long long keys[kKeyCount];
   __shared__ __align__(16) float vals[kValCount];
   __shared__ int part[3][kBlockQueryWarps];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -543,7 +550,7 @@ __global__ void __launch_bounds__(kBlockQueryWarps * 32)
   const int n_items = *work_count;
   for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
     const int64_t q = worklist[item];
-    for (int j = tid; j < kKeyCount / 4; j += kBlockQueryWarps * 32) reinterpret_cast<uint4*>(keys)[j] = make_uint4(0u, 0u, 0u, 0u);
+    for (int j = tid; j < kKeyCount / 2; j += kBlockQueryWarps * 32) reinterpret_cast<uint4*>(keys)[j] = make_uint4(0u, 0u, 0u, 0u);
     const double qx = __ldg(queries + 3 * q), qy = __ldg(queries + 3 * q + 1), qz = __ldg(queries + 3 * q + 2);
     const int64_t begin = offsets[q], end = counts ? begin + counts[q] : offsets[q + 1];
     double f[9];
@@ -586,6 +593,7 @@ __global__ void __launch_bounds__(kBlockQueryWarps * 32)
     for (int64_t base = begin; base < end; base += kBlockQueryWarps * 32) {  // block-uniform trip count (barriers inside)
       const int64_t i = base + tid;
       ShotDecision d;
+      unsigned long long key = 0;
       bool active = false;
       if (i < end) {
         const int s = __ldg(nbr + i * nbr_stride + nbr_word) & 0x7fffffff;
@@ -596,22 +604,23 @@ __global__ void __launch_bounds__(kBlockQueryWarps * 32)
           active = true;
           ++positive;
           const double rho = sqrt(d2);
-          const double X = cx * f[0] + cy * f[3] + cz * f[6];
-          const double Y = cx * f[1] + cy * f[4] + cz * f[7];
-          const double Z = cx * f[2] + cy * f[5] + cz * f[8];
+          const double X = frame_dot(cx, cy, cz, f[0], f[3], f[6]);
+          const double Y = frame_dot(cx, cy, cz, f[1], f[4], f[7]);
+          const double Z = frame_dot(cx, cy, cz, f[2], f[5], f[8]);
           double cosine = n.x * f[2] + n.y * f[5] + n.z * f[8];
           cosine = fmin(1.0, fmax(-1.0, cosine));
           d = shot_decide(X, Y, Z, cosine, rho, radius, inv_radius);
-          atomicMax(keys + kKeyOwn + d.own, d.key);
-          atomicMax(keys + kKeyCos + d.cos_nb, d.key);
-          atomicMax(keys + kKeyAz + d.az_nb, d.key);
+          key = shot_order_key(d.key, uint32_t(i - begin));
+          atomicMax(keys + kKeyOwn + d.own, key);
+          atomicMax(keys + kKeyCos + d.cos_nb, key);
+          atomicMax(keys + kKeyAz + d.az_nb, key);
         }
       }
       __syncthreads();
       if (active) {
-        const bool win_own = keys[kKeyOwn + d.own] == d.key;
-        const bool win_cos = keys[kKeyCos + d.cos_nb] == d.key;
-        const bool win_az = keys[kKeyAz + d.az_nb] == d.key;
+        const bool win_own = keys[kKeyOwn + d.own] == key;
+        const bool win_cos = keys[kKeyCos + d.cos_nb] == key;
+        const bool win_az = keys[kKeyAz + d.az_nb] == key;
         float a_az = 0.0f;
         if (win_own || win_az) a_az = shot_azimuth(d);
         if (win_own) {
@@ -640,16 +649,15 @@ __global__ void __launch_bounds__(kBlockQueryWarps * 32)
       for (int j = 0; j < kGroupRounds; ++j) {
         const int grp = lane + 32 * j;
         if (grp < kGroups) {
-          const uint4 ko = *reinterpret_cast<const uint4*>(keys + kKeyOwn + 4 * grp);
-          const uint4 kc = *reinterpret_cast<const uint4*>(keys + kKeyCos + 4 * grp);
-          const uint4 ka = *reinterpret_cast<const uint4*>(keys + kKeyAz + 4 * grp);
+          unsigned long long ko_[4], kc_[4], ka_[4];
+          load_keys4(keys + kKeyOwn + 4 * grp, ko_);
+          load_keys4(keys + kKeyCos + 4 * grp, kc_);
+          load_keys4(keys + kKeyAz + 4 * grp, ka_);
           const float4 vo = *reinterpret_cast<const float4*>(vals + kValOwn + 4 * grp);
           const float4 vr = *reinterpret_cast<const float4*>(vals + kValRad + 4 * grp);
           const float4 ve = *reinterpret_cast<const float4*>(vals + kValEl + 4 * grp);
           const float4 vc = *reinterpret_cast<const float4*>(vals + kValCos + 4 * grp);
           const float4 va = *reinterpret_cast<const float4*>(vals + kValAz + 4 * grp);
-          const uint32_t ko_[4] = {ko.x, ko.y, ko.z, ko.w}, kc_[4] = {kc.x, kc.y, kc.z, kc.w},
-                         ka_[4] = {ka.x, ka.y, ka.z, ka.w};
           const float vo_[4] = {vo.x, vo.y, vo.z, vo.w}, vr_[4] = {vr.x, vr.y, vr.z, vr.w},
                       ve_[4] = {ve.x, ve.y, ve.z, ve.w}, vc_[4] = {vc.x, vc.y, vc.z, vc.w},
                       va_[4] = {va.x, va.y, va.z, va.w};
@@ -1195,9 +1203,9 @@ static int launch_descriptor(sf_grid* g, const double* queries, int64_t nq, doub
       SF_CUDA(launch(shot_fast_kernel<float, true, 8, 2>, fo, 8, 2));
     }
   }
-  // exact kernel, persistent-style: 148 SMs x 5 resident blocks (44 KB shared memory each), capped by the work
+  // exact kernel, persistent-style: 148 SMs x 3 resident blocks (62 KB shared memory each), capped by the work
   const int64_t blocks_needed = (nq + kShotWarpsPerBlock - 1) / kShotWarpsPerBlock;
-  const unsigned blocks = unsigned(blocks_needed < 148 * 5 ? blocks_needed : 148 * 5);
+  const unsigned blocks = unsigned(blocks_needed < 148 * 3 ? blocks_needed : 148 * 3);
   const int32_t* wl = exact_only ? nullptr : worklist;
   const int32_t* nbr = static_cast<const int32_t*>(list);
   const int stride = records ? 4 : 1;

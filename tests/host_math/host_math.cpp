@@ -39,6 +39,14 @@ long hm_dsteqr3_static_vs_generic(const double* d3, const double* e2, long n) {
 
 int hm_azimuth_octant(double x, double y) { return azimuth_octant(x, y); }
 
+double hm_acos_half_pi_max() { return kAcosHalfPiMax; }
+
+// local = rel @ lrf for k offsets (rel: k x 3, lrf9 row-major, columns [x y z]) as the float64 kernels round it
+void hm_frame_local(const double* rel, long k, const double* f, double* local) {
+  for (long i = 0; i < k; ++i)
+    for (int j = 0; j < 3; ++j) local[3 * i + j] = frame_dot(rel[3 * i], rel[3 * i + 1], rel[3 * i + 2], f[j], f[3 + j], f[6 + j]);
+}
+
 // Mirrors shot_lrf_kernel: lrf9 row-major, columns [x y z].
 void hm_lrf(const double* point, const double* nbrs, int k, double radius, double* lrf9) {
   if (k == 0) {
@@ -77,12 +85,13 @@ void hm_lrf(const double* point, const double* nbrs, int k, double radius, doubl
 // then value pass), atomicMax replaced by a sequential max.
 void hm_shot_descriptor(const double* point, const double* nbrs, const double* normals, int k, double radius,
                         const double* f, int normalize, int min_nb, float* out352) {
-  std::vector<uint32_t> keys(kKeyCount, 0u);
+  std::vector<uint64_t> keys(kKeyCount, 0u);
   std::vector<float> vals(kValCount, 0.0f);
   int positive = 0;
   const double inv_radius = 1.0 / radius;
   for (int base = 0; base < k; base += 32) {
     ShotDecision d[32];
+    uint64_t key[32];
     bool active[32];
     for (int lane = 0; lane < 32; ++lane) {
       active[lane] = false;
@@ -94,21 +103,22 @@ void hm_shot_descriptor(const double* point, const double* nbrs, const double* n
       active[lane] = true;
       ++positive;
       const double rho = sqrt(d2);
-      const double X = cx * f[0] + cy * f[3] + cz * f[6];
-      const double Y = cx * f[1] + cy * f[4] + cz * f[7];
-      const double Z = cx * f[2] + cy * f[5] + cz * f[8];
+      const double X = frame_dot(cx, cy, cz, f[0], f[3], f[6]);
+      const double Y = frame_dot(cx, cy, cz, f[1], f[4], f[7]);
+      const double Z = frame_dot(cx, cy, cz, f[2], f[5], f[8]);
       double cosine = normals[3 * i] * f[2] + normals[3 * i + 1] * f[5] + normals[3 * i + 2] * f[8];
       cosine = fmin(1.0, fmax(-1.0, cosine));
       d[lane] = shot_decide(X, Y, Z, cosine, rho, radius, inv_radius);
-      if (d[lane].key > keys[kKeyOwn + d[lane].own]) keys[kKeyOwn + d[lane].own] = d[lane].key;
-      if (d[lane].key > keys[kKeyCos + d[lane].cos_nb]) keys[kKeyCos + d[lane].cos_nb] = d[lane].key;
-      if (d[lane].key > keys[kKeyAz + d[lane].az_nb]) keys[kKeyAz + d[lane].az_nb] = d[lane].key;
+      key[lane] = shot_order_key(d[lane].key, uint32_t(i));
+      if (key[lane] > keys[kKeyOwn + d[lane].own]) keys[kKeyOwn + d[lane].own] = key[lane];
+      if (key[lane] > keys[kKeyCos + d[lane].cos_nb]) keys[kKeyCos + d[lane].cos_nb] = key[lane];
+      if (key[lane] > keys[kKeyAz + d[lane].az_nb]) keys[kKeyAz + d[lane].az_nb] = key[lane];
     }
     for (int lane = 0; lane < 32; ++lane) {
       if (!active[lane]) continue;
       const ShotDecision& e = d[lane];
-      const bool win_own = keys[kKeyOwn + e.own] == e.key, win_cos = keys[kKeyCos + e.cos_nb] == e.key,
-                 win_az = keys[kKeyAz + e.az_nb] == e.key;
+      const bool win_own = keys[kKeyOwn + e.own] == key[lane], win_cos = keys[kKeyCos + e.cos_nb] == key[lane],
+                 win_az = keys[kKeyAz + e.az_nb] == key[lane];
       float a_az = 0.0f;
       if (win_own || win_az) a_az = shot_azimuth(e);
       if (win_own) {
@@ -125,7 +135,7 @@ void hm_shot_descriptor(const double* point, const double* nbrs, const double* n
   double sq = 0.0;
   float v[kShotLen];
   for (int g = 0; g < kShotLen / 4; ++g) {  // four bins of one (cosine, azimuth) cell at a time, as the kernel does
-    const uint32_t* k = keys.data() + 4 * g;
+    const uint64_t* k = keys.data() + 4 * g;
     const float* x = vals.data() + 4 * g;
     shot_bin_group_compact(k + kKeyOwn, k + kKeyCos, k + kKeyAz, x + kValOwn, x + kValRad, x + kValEl, x + kValCos,
                            x + kValAz, v + 4 * g);

@@ -415,3 +415,91 @@ def test_spfh_counts_match_oracle(hm, cloud, n_bins, decorrelated):
         )
         mismatched += int(not np.array_equal(hist, np.rint(want).astype(np.int32)))
     assert mismatched == 0
+
+
+# ---- planar neighbourhoods and hand-built boundary probes (oracle/shot_probes.py) -----------------------------------
+def test_arccos_half_pi_window_is_numpys(hm):
+    """sf_math.cuh::kAcosHalfPiMax is the largest Z / rho > 0 for which np.arccos returns exactly np.pi / 2 (the
+    reference then writes `lower` = 0 although the neighbour is binned in the upper half)."""
+    from oracle import shot_probes
+
+    hm.hm_acos_half_pi_max.restype = ctypes.c_double
+    lo, hi = 1e-18, 1e-15  # arccos(lo) == pi/2 > arccos(hi): bisect on the doubles between them
+    assert np.arccos(lo) == np.pi / 2 and np.arccos(hi) < np.pi / 2
+    lo_i, hi_i = np.float64(lo).view(np.int64), np.float64(hi).view(np.int64)
+    while hi_i - lo_i > 1:
+        mid = (lo_i + hi_i) // 2
+        if np.arccos(np.int64(mid).view(np.float64)) == np.pi / 2:
+            lo_i = mid
+        else:
+            hi_i = mid
+    window = float(np.int64(lo_i).view(np.float64))
+    assert window == hm.hm_acos_half_pi_max() == shot_probes.A_HALF_PI_MAX
+    assert np.arccos(np.nextafter(window, 1.0)) < np.pi / 2
+    assert np.arccos(-window) > np.pi / 2  # below zero the window is narrower, and Z <= 0 takes the other branch
+
+
+def test_numpy_matmul_rounds_like_frame_dot(hm):
+    """The oracle's `rel @ lrf` equals sf_math.cuh::frame_dot bit for bit (fused multiply-adds, k = 0, 1, 2): on a
+    plane the sign of Z is rounding noise and picks the elevation bin."""
+    hm.hm_frame_local.argtypes = [DP, ctypes.c_long, DP, DP]
+    rng = np.random.default_rng(31)
+    n = 20000
+    xy = rng.uniform(0, 1, (n, 2))
+    for rel in (rng.normal(size=(n, 3)), np.column_stack([xy, 0.3 * xy[:, 0] - 0.2 * xy[:, 1]]) - [0.5, 0.5, 0.05]):
+        rel = np.ascontiguousarray(rel)
+        frame = shot_oracle.local_reference_frame(np.zeros(3), rel[:200], 0.1)
+        got = np.zeros_like(rel)
+        hm.hm_frame_local(_p(rel), n, _p(np.ascontiguousarray(frame)), _p(got))
+        assert np.array_equal(got, rel @ frame)
+
+
+def _host_row(hm, point, nbrs, normals, radius, frame, normalize=True, min_nb=10):
+    got = np.zeros(352, dtype=np.float32)
+    hm.hm_shot_descriptor(
+        _p(np.ascontiguousarray(point)), _p(np.ascontiguousarray(nbrs)), _p(np.ascontiguousarray(normals)),
+        nbrs.shape[0], radius, _p(np.ascontiguousarray(frame)), int(normalize), min_nb, got.ctypes.data_as(FP))
+    return got.astype(np.float64)
+
+
+@pytest.mark.parametrize("tilt", [(0.0, 0.0), (0.3, -0.2)])
+def test_shot_planar_neighbourhoods_match_oracle(hm, tilt):
+    """On a plane every Z is 0 or rounding noise: the float64 path (what the fast kernel hands such queries to) must
+    follow the oracle there too, including Z / rho inside the arccos window (sf_math.cuh::kAcosHalfPiMax)."""
+    rng = np.random.default_rng(7)
+    n = 20000
+    xy = rng.uniform(0, 1, (n, 2))
+    pts = np.column_stack([xy, tilt[0] * xy[:, 0] + tilt[1] * xy[:, 1]])
+    normals = np.array([-tilt[0], -tilt[1], 1.0]) + 0.1 * rng.normal(size=(n, 3))
+    normals /= np.linalg.norm(normals, axis=1, keepdims=True)
+    radius = 5.0 / np.sqrt(n)
+    tree = KDTree(pts)
+    errs = []
+    for i in range(0, n, 67):
+        nb = tree.query_radius(pts[i : i + 1], radius)[0]
+        lrf = shot_oracle.local_reference_frame(pts[i], pts[nb], radius)
+        want = shot_oracle.shot_descriptor(pts[i], pts[nb], normals[nb], radius, lrf, True, 10)
+        errs.append(float(rel_l2(_host_row(hm, pts[i], pts[nb], normals[nb], radius, lrf), want)))
+    errs = np.array(errs)
+    print(f"plane {tilt}: {errs.shape[0]} rows, median {np.median(errs):.1e}, max {errs.max():.1e}")
+    assert errs.max() <= 1e-5
+
+
+def test_shot_boundary_probes_match_oracle(hm):
+    """oracle/shot_probes.py: a neighbour on (and 1 ulp .. 1e-5 r off) every decision boundary, frames that copy
+    coordinates exactly: the float64 path equals the oracle to 1e-5 on every row."""
+    from oracle import shot_probes
+
+    pts, normals, queries, frames, kinds = shot_probes.probe_set()
+    radius = shot_probes.RADIUS
+    tree = KDTree(pts)
+    worst = {}
+    for q, frame, kind in zip(queries, frames, kinds):
+        nb = tree.query_radius(q[None], radius)[0]
+        for normalize in (True, False):
+            want = shot_oracle.shot_descriptor(q, pts[nb], normals[nb], radius, frame, normalize, 10)
+            assert want.any()
+            err = float(rel_l2(_host_row(hm, q, pts[nb], normals[nb], radius, frame, normalize), want))
+            worst[kind] = max(worst.get(kind, 0.0), err)
+    print({k: f"{v:.1e}" for k, v in worst.items()})
+    assert max(worst.values()) <= 1e-5, worst
