@@ -1,10 +1,10 @@
 """
 Tuning / attribution run for the C2 SHOT step on one B200 (not part of the product, not a benchmark line):
-per-stage CUDA-event times of the fused single-scale driver for each variant of the float32 descriptor kernel
-(SF_FAST_SHAPE = resident blocks per SM it is compiled for), the number of queries it hands to the float64
-kernel, and its rows against the float64 kernel's (SF_SHOT_EXACT=1).
+per-stage CUDA-event times of the fused single-scale driver, by default and under each environment of --envs,
+the number of queries the float32 descriptor kernel hands to the float64 kernel, and its rows against the float64
+kernel's (SF_SHOT_EXACT=1).
 
-    python scripts/tune_shot.py [--variants 43,33,34,42,44] [--steps 12] [--n 1000000]
+    python scripts/tune_shot.py [--envs NAME=VALUE+NAME=VALUE,...] [--steps 12] [--n 1000000]
 """
 
 from __future__ import annotations
@@ -22,8 +22,7 @@ sys.path.insert(0, ROOT)
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--variants", default="82,73,102,63")
-    ap.add_argument("--envs", default="", help="further variants, each a +-joined list of NAME=VALUE, separated by commas")
+    ap.add_argument("--envs", default="", help="variants besides the default, each a +-joined list of NAME=VALUE, separated by commas")
     ap.add_argument("--no-profile", action="store_true", help="step times only: no CUDA events between the kernels")
     ap.add_argument("--steps", type=int, default=12)
     ap.add_argument("--n", type=int, default=1_000_000)
@@ -78,7 +77,7 @@ def main():
 
     exact = run("exact", {"SF_SHOT_EXACT": "1"})
     exact_norm = exact.double().norm(dim=1).clamp_min(1e-300)
-    variants = [(v, {"SF_FAST_SHAPE": v}) for v in args.variants.split(",") if v]
+    variants = [("default", {})]
     variants += [(e, dict(kv.split("=") for kv in e.split("+"))) for e in args.envs.split(",") if e]
     for v, env in variants:
         got = run(f"fast_{v}", env)

@@ -161,6 +161,28 @@ SF_HD ShotDecision shot_decide(double X, double Y, double Z, double cosine, doub
   return d;
 }
 
+// The float64 step of one neighbour: offset c = p - q and normal n in the frame f (row-major, columns [x y z]).
+SF_HD ShotDecision shot_decide_in_frame(double cx, double cy, double cz, double nx, double ny, double nz,
+                                        const double f[9], double rho, double radius, double inv_radius) {
+  const double X = frame_dot(cx, cy, cz, f[0], f[3], f[6]);
+  const double Y = frame_dot(cx, cy, cz, f[1], f[4], f[7]);
+  const double Z = frame_dot(cx, cy, cz, f[2], f[5], f[8]);
+  double cosine = nx * f[2] + ny * f[5] + nz * f[8];
+  cosine = fmin(1.0, fmax(-1.0, cosine));
+  return shot_decide(X, Y, Z, cosine, rho, radius, inv_radius);
+}
+
+// The local reference frame from the raw eigenvectors x, z and the sign votes of shot.py:40-45 (an axis is negated when
+// strictly more neighbours project negatively on it than not), y = z cross x in float64. f: row-major, columns [x y z].
+SF_HD void shot_frame(const double x_raw[3], const double z_raw[3], bool flip_x, bool flip_z, double f[9]) {
+  const double sx = flip_x ? -1.0 : 1.0, sz = flip_z ? -1.0 : 1.0;  // (exact negation)
+  const double x[3] = {sx * x_raw[0], sx * x_raw[1], sx * x_raw[2]}, z[3] = {sz * z_raw[0], sz * z_raw[1], sz * z_raw[2]};
+  const double y[3] = {z[1] * x[2] - z[2] * x[1], z[2] * x[0] - z[0] * x[2], z[0] * x[1] - z[1] * x[0]};
+  f[0] = x[0]; f[1] = y[0]; f[2] = z[0];
+  f[3] = x[1]; f[4] = y[1]; f[5] = z[1];
+  f[6] = x[2]; f[7] = y[2]; f[8] = z[2];
+}
+
 // ---- step 2: the two transcendental weights, float32 (continuous in their inputs) ---------------------------------
 // elevation (shot.py:142-171): phi < pi/2 <=> Z > 0 (see DESIGN.md), except in the window of kAcosHalfPiMax
 SF_HD void shot_elevation(const ShotDecision& d, float& own_vol, float& other_vol) {
@@ -416,15 +438,30 @@ SF_HD bool shot_keys_ambiguous(uint32_t a, uint32_t b, uint32_t margin) {
 // Keys are raised with a native 64-bit atomicMax; after a barrier the lane whose key is (still) the slot's key stores
 // its values. The key is the 32-bit distance key, then the neighbour's position in the query's list: keys are unique
 // inside a query, so two neighbours at the same distance (exact ties, or distances within radius * 2^-32) cannot both
-// win a slot, and the later one in the list wins whatever the schedule — the warp kernel, the block kernel and a
-// repeated call give the same row. (The reference breaks such ties by its unstable argsort: the tie itself stays an
-// exemption, DESIGN.md §2.)
+// win a slot, and the later one in the list wins whatever the schedule — every run and every thread count gives the
+// same row. (The reference breaks such ties by its unstable argsort: the tie itself stays an exemption, DESIGN.md §2.)
 SF_HD uint64_t shot_order_key(uint32_t distance_key, uint32_t position) {
   return (uint64_t(distance_key) << 32) | position;
 }
 constexpr int kKeyOwn = 0, kKeyCos = kShotLen, kKeyAz = 2 * kShotLen, kKeyCount = 3 * kShotLen;
 constexpr int kValOwn = 0, kValRad = kShotLen, kValEl = 2 * kShotLen, kValCos = 3 * kShotLen, kValAz = 4 * kShotLen,
               kValCount = 5 * kShotLen;
+
+// The values of a neighbour that holds (still, after the barrier) the key of its own-bin, statement-1 and / or
+// statement-9 slot; only a winner pays for the transcendental weights it needs.
+SF_HD void shot_store_winner(const ShotDecision& d, bool win_own, bool win_cos, bool win_az, float* vals) {
+  float a_az = 0.0f;
+  if (win_own || win_az) a_az = shot_azimuth(d);
+  if (win_own) {
+    float own_vol, other_vol;
+    shot_elevation(d, own_vol, other_vol);
+    vals[kValOwn + d.own] = (1.0f - d.a_cos) + d.own_shell + own_vol + (1.0f - a_az);
+    vals[kValRad + d.own] = d.other_shell;
+    vals[kValEl + d.own] = other_vol;
+  }
+  if (win_cos) vals[kValCos + d.cos_nb] = d.a_cos;
+  if (win_az) vals[kValAz + d.az_nb] = a_az;
+}
 
 template <typename Key>
 SF_HD float shot_bin_value_compact(const Key* keys, const float* vals, int flat) {

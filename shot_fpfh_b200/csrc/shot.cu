@@ -1,12 +1,12 @@
-// Kernel group S: SHOT local reference frames and 352-bin descriptors, one warp per query point.
-//   S1 shot_lrf_kernel        <- get_local_rf, shot.py:16-48 (fan-out shot_parallelization.py:46-84)
-//   S2 shot_descriptor_kernel <- compute_single_shot_descriptor, shot.py:175-306 (fan-out :86-133)
+// Kernel group S: SHOT local reference frames and 352-bin descriptors.
+//   S1 shot_lrf_kernel <- get_local_rf, shot.py:16-48 (fan-out shot_parallelization.py:46-84)
+//   S2 shot_fast_kernel, shot_descriptor_block_kernel <- compute_single_shot_descriptor, shot.py:175-306 (fan-out :86-133)
 //
 // S2 implements the reference's actual semantics (SURVEY.md F1 / Appendix A): its ten `descriptor[idx] += v`
 // statements are buffered NumPy fancy-index updates, so per statement and per bin only the neighbour with the
-// largest distance that addresses the bin contributes (even with value 0). Each warp owns compact winner tables in
-// shared memory (sf_math.cuh: three uint64 key tables raised with the native 64-bit atomicMax, five float value
-// tables written by the lanes that still hold a slot's key after a warp barrier); bins then sum their statements.
+// largest distance that addresses the bin contributes (even with value 0). The float64 kernel keeps compact winner
+// tables in shared memory (sf_math.cuh: three uint64 key tables raised with the native 64-bit atomicMax, five float
+// value tables written by the threads that still hold a slot's key after a barrier); bins then sum their statements.
 #include <cub/cub.cuh>
 
 #include "sf_common.cuh"
@@ -128,8 +128,8 @@ __global__ void __launch_bounds__(256)
     return;
   }
   const double qx = __ldg(queries + 3 * q), qy = __ldg(queries + 3 * q + 1), qz = __ldg(queries + 3 * q + 2);
-  double x[3] = {out[0], out[1], out[2]}, z[3] = {out[3], out[4], out[5]};
-  // sign votes (shot.py:40-45): flip when strictly more neighbours project negatively than non-negatively
+  const double x[3] = {out[0], out[1], out[2]}, z[3] = {out[3], out[4], out[5]};
+  // sign votes (shot.py:40-45)
   int neg_x = 0, neg_z = 0;
   for (int64_t i = begin + lane; i < end; i += 32) {
     const double4 p = load_pt(g.pts + __ldg(nbr + i));
@@ -140,14 +140,12 @@ __global__ void __launch_bounds__(256)
   neg_x = warp_sum(neg_x);
   neg_z = warp_sum(neg_z);
   const int k_all = int(end - begin);
-  if (neg_x > k_all - neg_x) { x[0] = -x[0]; x[1] = -x[1]; x[2] = -x[2]; }
-  if (neg_z > k_all - neg_z) { z[0] = -z[0]; z[1] = -z[1]; z[2] = -z[2]; }
-  const double y[3] = {z[1] * x[2] - z[2] * x[1], z[2] * x[0] - z[0] * x[2], z[0] * x[1] - z[1] * x[0]};
+  double f[9];
+  shot_frame(x, z, neg_x > k_all - neg_x, neg_z > k_all - neg_z, f);
   __syncwarp();  // every lane has read the axes before the frame overwrites them
-  if (lane < 3) {  // row `lane` of the matrix whose columns are [x y z] (selects, not indexing: stays in registers)
-    out[3 * lane + 0] = lane == 0 ? x[0] : (lane == 1 ? x[1] : x[2]);
-    out[3 * lane + 1] = lane == 0 ? y[0] : (lane == 1 ? y[1] : y[2]);
-    out[3 * lane + 2] = lane == 0 ? z[0] : (lane == 1 ? z[1] : z[2]);
+  if (lane < 3) {  // row `lane` of the frame (selects, not indexing: stays in registers)
+#pragma unroll
+    for (int c = 0; c < 3; ++c) out[3 * lane + c] = lane == 0 ? f[c] : (lane == 1 ? f[3 + c] : f[6 + c]);
   }
 }
 
@@ -330,19 +328,21 @@ __global__ void __launch_bounds__(256)
   }
 }
 
-// ---- S2 ----------------------------------------------------------------------------------------------------
-// Per warp: uint64 keys[3][352] + float vals[5][352] = 15 488 B of shared memory (sf_math.cuh, "winner tables,
-// compact form"). Per 32 neighbours: (a) float64 decisions, (b) three native 64-bit atomicMax on the key tables,
-// (c) warp barrier, (d) the lanes that hold a slot's key compute the transcendental weights they need (only winners
-// pay for acosf / atan2f) and store their values. After the last neighbour each lane assembles 11 bins.
-constexpr int kShotWarpsPerBlock = 4;
+// ---- S2, float64: a BLOCK per query -----------------------------------------------------------------------------------
+// For the queries the fast kernel below hands over (a few hundred: 603 of 102 336 at C2; one warp per query walking its
+// neighbours 32 at a time was 15-17 us of latency at the end of the step) and for every query under SF_SHOT_EXACT=1.
+// uint64 keys[3][352] + float vals[5][352] = 15 488 B of shared memory per block (sf_math.cuh, "winner tables, compact
+// form"). The four warps take the batches of 32 neighbours in turn (the sign votes as well). Per 128 neighbours:
+// (a) float64 decisions, (b) three native 64-bit atomicMax on the key tables, (c) block barrier, (d) the threads that
+// hold a slot's key compute the transcendental weights they need (only winners pay for acosf / atan2f) and store their
+// values. After the last neighbour warp 0 assembles the 352 bins.
+constexpr int kBlockQueryWarps = 4;
 
 // Four consecutive 64-bit keys (32-byte aligned) as two 16-byte shared-memory reads.
 __device__ __forceinline__ void load_keys4(const unsigned long long* k, unsigned long long out[4]) {
   const ulonglong2 a = reinterpret_cast<const ulonglong2*>(k)[0], b = reinterpret_cast<const ulonglong2*>(k)[1];
   out[0] = a.x; out[1] = a.y; out[2] = b.x; out[3] = b.y;
 }
-constexpr int kShotSmemPerWarp = kKeyCount * 8 + kValCount * 4;
 
 // 352 * sizeof(OutT) is a multiple of 16, so every row and every group of four bins is 16-byte aligned
 __device__ __forceinline__ void store_group(float* p, float a, float b, float c, float d) {
@@ -354,202 +354,34 @@ __device__ __forceinline__ void store_group(double* p, float a, float b, float c
 }
 
 template <typename OutT>
-__global__ void __launch_bounds__(kShotWarpsPerBlock * 32, 5)
-    shot_descriptor_kernel(GridView g, const double* __restrict__ queries, int64_t nq, double radius,
-                           const int64_t* __restrict__ offsets, const int32_t* __restrict__ counts,
-                           const int32_t* __restrict__ nbr, double* __restrict__ lrf, int fuse_votes, int min_nb,
-                           int normalize, OutT* __restrict__ out, const int32_t* __restrict__ worklist,
-                           const int32_t* __restrict__ work_count, int nbr_stride,
-                           const int32_t* __restrict__ status) {
-  if (status != nullptr && *status != 0) return;
-  // counts == nullptr: classic CSR, neighbours of q are nbr[offsets[q] .. offsets[q+1]). Otherwise a padded list:
-  // nbr[offsets[q] .. offsets[q] + counts[q]) (the fused single-scale driver).
-  // fuse_votes: lrf[9q + 0..5] holds the RAW eigenvectors (x, z) from lrf_eigen_kernel; the sign votes of
-  // shot.py:40-45 run here (the second pass over the same neighbours then hits L1) and the final frame is written
-  // back to lrf[9q + 0..8].
-  // worklist != nullptr: only the queries worklist[0 .. *work_count) (the ones shot_fast_kernel handed over).
-  // nbr_stride = 4: `nbr` is the fused driver's list of 16-byte entries (float32 offset, position | flag << 31), the
-  // position is word 3 of an entry and offsets / counts are in entries; the flag (neighbour at distance 0) is masked:
-  // this kernel decides that in float64 itself. nbr_stride = 1: plain int32 positions.
-  extern __shared__ uint32_t table_mem[];
-  const int lane = threadIdx.x & 31;
-  const int warp = threadIdx.x >> 5;
-  unsigned long long* keys = reinterpret_cast<unsigned long long*>(table_mem + warp * (kShotSmemPerWarp / 4));
-  float* vals = reinterpret_cast<float*>(keys + kKeyCount);
-  const int64_t warps_total = int64_t(gridDim.x) * kShotWarpsPerBlock;
-  const double inv_radius = 1.0 / radius;
-  const int nbr_word = nbr_stride - 1;
-  const int64_t n_items = worklist != nullptr ? int64_t(*work_count) : nq;
-  for (int64_t item = blockIdx.x * int64_t(kShotWarpsPerBlock) + warp; item < n_items; item += warps_total) {
-    const int64_t q = worklist != nullptr ? int64_t(worklist[item]) : item;
-    // values are gated by their keys: only the keys are cleared (16 bytes per lane and store)
-    for (int j = lane; j < kKeyCount / 2; j += 32) reinterpret_cast<uint4*>(keys)[j] = make_uint4(0u, 0u, 0u, 0u);
-    const double qx = __ldg(queries + 3 * q), qy = __ldg(queries + 3 * q + 1), qz = __ldg(queries + 3 * q + 2);
-    const int64_t begin = offsets[q], end = counts ? begin + counts[q] : offsets[q + 1];
-    double f[9];
-    if (!fuse_votes) {
-#pragma unroll
-      for (int k = 0; k < 9; ++k) f[k] = lrf[9 * q + k];
-    } else if (end == begin) {
-#pragma unroll
-      for (int k = 0; k < 9; ++k) f[k] = (k % 4 == 0) ? 1.0 : 0.0;  // shot.py:24-25
-      __syncwarp();
-      if (lane < 9) lrf[9 * q + lane] = (lane % 4 == 0) ? 1.0 : 0.0;
-    } else {
-      double x[3] = {lrf[9 * q], lrf[9 * q + 1], lrf[9 * q + 2]}, z[3] = {lrf[9 * q + 3], lrf[9 * q + 4], lrf[9 * q + 5]};
-      int neg_x = 0, neg_z = 0;
-      for (int64_t i = begin + lane; i < end; i += 32) {
-        const double4 p = load_pt(g.pts + (__ldg(nbr + i * nbr_stride + nbr_word) & 0x7fffffff));
-        const double cx = p.x - qx, cy = p.y - qy, cz = p.z - qz;
-        neg_x += (cx * x[0] + cy * x[1] + cz * x[2]) < 0.0;
-        neg_z += (cx * z[0] + cy * z[1] + cz * z[2]) < 0.0;
-      }
-      neg_x = warp_sum(neg_x);
-      neg_z = warp_sum(neg_z);
-      const int k_all = int(end - begin);
-      if (neg_x > k_all - neg_x) { x[0] = -x[0]; x[1] = -x[1]; x[2] = -x[2]; }
-      if (neg_z > k_all - neg_z) { z[0] = -z[0]; z[1] = -z[1]; z[2] = -z[2]; }
-      const double y[3] = {z[1] * x[2] - z[2] * x[1], z[2] * x[0] - z[0] * x[2], z[0] * x[1] - z[1] * x[0]};
-#pragma unroll
-      for (int a = 0; a < 3; ++a) { f[3 * a] = x[a]; f[3 * a + 1] = y[a]; f[3 * a + 2] = z[a]; }
-      __syncwarp();  // every lane has read the raw axes before the frame overwrites them
-      if (lane == 0) {
-#pragma unroll
-        for (int k = 0; k < 9; ++k) lrf[9 * q + k] = f[k];
-      }
-    }
-    int positive = 0;
-    // software pipeline: the gathers of the lane's NEXT neighbour are issued before the current one is processed
-    // (the neighbour INDEX runs one round further ahead still, so that a gather never waits for its address)
-    int64_t i = begin + lane;
-    double4 p_next = make_double4(0, 0, 0, 0), n_next = p_next;
-    int s_after = 0;
-    if (i < end) {
-      const int s = __ldg(nbr + i * nbr_stride + nbr_word) & 0x7fffffff;
-      p_next = load_pt(g.pts + s);
-      n_next = load_pt(g.nrm + s);
-    }
-    if (i + 32 < end) s_after = __ldg(nbr + (i + 32) * nbr_stride + nbr_word) & 0x7fffffff;
-    __syncwarp();
-    for (int64_t base = begin; base < end; base += 32, i += 32) {  // warp-uniform trip count (barriers inside)
-      const double4 p = p_next, n = n_next;
-      if (i + 32 < end) {
-        const int s = s_after;
-        p_next = load_pt(g.pts + s);
-        n_next = load_pt(g.nrm + s);
-        if (i + 64 < end) s_after = __ldg(nbr + (i + 64) * nbr_stride + nbr_word) & 0x7fffffff;
-      }
-      ShotDecision d;
-      unsigned long long key = 0;
-      bool active = false;
-      if (i < end) {
-        const double cx = p.x - qx, cy = p.y - qy, cz = p.z - qz;
-        const double d2 = rdist3(cx, cy, cz);
-        if (d2 > 0.0) {  // shot.py:213: neighbours at distance 0 (the query itself, duplicates) are dropped
-          active = true;
-          ++positive;
-          const double rho = sqrt(d2);
-          const double X = frame_dot(cx, cy, cz, f[0], f[3], f[6]);
-          const double Y = frame_dot(cx, cy, cz, f[1], f[4], f[7]);
-          const double Z = frame_dot(cx, cy, cz, f[2], f[5], f[8]);
-          double cosine = n.x * f[2] + n.y * f[5] + n.z * f[8];
-          cosine = fmin(1.0, fmax(-1.0, cosine));
-          d = shot_decide(X, Y, Z, cosine, rho, radius, inv_radius);
-          key = shot_order_key(d.key, uint32_t(i - begin));
-          atomicMax(keys + kKeyOwn + d.own, key);
-          atomicMax(keys + kKeyCos + d.cos_nb, key);
-          atomicMax(keys + kKeyAz + d.az_nb, key);
-        }
-      }
-      __syncwarp();
-      if (active) {
-        const bool win_own = keys[kKeyOwn + d.own] == key;
-        const bool win_cos = keys[kKeyCos + d.cos_nb] == key;
-        const bool win_az = keys[kKeyAz + d.az_nb] == key;
-        float a_az = 0.0f;
-        if (win_own || win_az) a_az = shot_azimuth(d);
-        if (win_own) {
-          float own_vol, other_vol;
-          shot_elevation(d, own_vol, other_vol);
-          vals[kValOwn + d.own] = (1.0f - d.a_cos) + d.own_shell + own_vol + (1.0f - a_az);
-          vals[kValRad + d.own] = d.other_shell;
-          vals[kValEl + d.own] = other_vol;
-        }
-        if (win_cos) vals[kValCos + d.cos_nb] = d.a_cos;
-        if (win_az) vals[kValAz + d.az_nb] = a_az;
-      }
-      __syncwarp();  // the stores above are ordered before the next round's key updates
-    }
-    positive = warp_sum(positive);
-    // assembly: lane handles the groups {lane, lane + 32, lane + 64} of four consecutive bins (one (cosine, azimuth)
-    // cell: the radial / elevation partners are inside the group) -> eight 16-byte table reads and one 16-byte
-    // store per group
-    constexpr int kGroups = kShotLen / 4, kGroupRounds = (kGroups + 31) / 32;
-    float v[kGroupRounds][4];
-    double sq = 0.0;
-#pragma unroll
-    for (int j = 0; j < kGroupRounds; ++j) {
-      const int grp = lane + 32 * j;
-      if (grp < kGroups) {
-        unsigned long long ko_[4], kc_[4], ka_[4];
-        load_keys4(keys + kKeyOwn + 4 * grp, ko_);
-        load_keys4(keys + kKeyCos + 4 * grp, kc_);
-        load_keys4(keys + kKeyAz + 4 * grp, ka_);
-        const float4 vo = *reinterpret_cast<const float4*>(vals + kValOwn + 4 * grp);
-        const float4 vr = *reinterpret_cast<const float4*>(vals + kValRad + 4 * grp);
-        const float4 ve = *reinterpret_cast<const float4*>(vals + kValEl + 4 * grp);
-        const float4 vc = *reinterpret_cast<const float4*>(vals + kValCos + 4 * grp);
-        const float4 va = *reinterpret_cast<const float4*>(vals + kValAz + 4 * grp);
-        const float vo_[4] = {vo.x, vo.y, vo.z, vo.w}, vr_[4] = {vr.x, vr.y, vr.z, vr.w},
-                    ve_[4] = {ve.x, ve.y, ve.z, ve.w}, vc_[4] = {vc.x, vc.y, vc.z, vc.w},
-                    va_[4] = {va.x, va.y, va.z, va.w};
-        shot_bin_group_compact(ko_, kc_, ka_, vo_, vr_, ve_, vc_, va_, v[j]);
-#pragma unroll
-        for (int t = 0; t < 4; ++t) sq += double(v[j][t]) * double(v[j][t]);
-      }
-    }
-    sq = warp_sum(sq);
-    const double norm = sqrt(sq);
-    // shot.py:212, :301-306: zero row when too few neighbours or a zero norm
-    const bool keep = positive > min_nb && norm > 0.0;
-    const float inv = keep ? (normalize ? float(1.0 / norm) : 1.0f) : 0.0f;
-    OutT* row = out + q * kShotLen;
-#pragma unroll
-    for (int j = 0; j < kGroupRounds; ++j) {
-      const int grp = lane + 32 * j;
-      if (grp < kGroups) store_group(row + 4 * grp, v[j][0] * inv, v[j][1] * inv, v[j][2] * inv, v[j][3] * inv);
-    }
-    __syncwarp();  // all lanes have read the tables before the next query clears the keys
-  }
-}
-
-
-// ---- S2, the same float64 kernel with a BLOCK per query -----------------------------------------------------------
-// For the work list of the fast kernel: a few hundred queries (603 of 102 336 at C2), i.e. one warp on each SM walking
-// its query's neighbours 32 at a time — 15-17 us of pure latency at the end of the step. Here the four warps of a block
-// share one set of winner tables and take the batches of 32 neighbours in turn (the sign votes as well), with block
-// barriers where the warp kernel has warp barriers; the assembly of the 352 bins is warp 0's, in the warp kernel's
-// order of additions, so the rows are the warp kernel's bit for bit (the tests compare the two kernels).
-constexpr int kBlockQueryWarps = 4;
-
-template <typename OutT>
 __global__ void __launch_bounds__(kBlockQueryWarps * 32)
-    shot_descriptor_block_kernel(GridView g, const double* __restrict__ queries, double radius,
+    shot_descriptor_block_kernel(GridView g, const double* __restrict__ queries, int64_t nq, double radius,
                                  const int64_t* __restrict__ offsets, const int32_t* __restrict__ counts,
                                  const int32_t* __restrict__ nbr, double* __restrict__ lrf, int fuse_votes, int min_nb,
                                  int normalize, OutT* __restrict__ out, const int32_t* __restrict__ worklist,
                                  const int32_t* __restrict__ work_count, int nbr_stride,
                                  const int32_t* __restrict__ status) {
   if (status != nullptr && *status != 0) return;
+  // counts == nullptr: classic CSR, neighbours of q are nbr[offsets[q] .. offsets[q+1]). Otherwise a padded list:
+  // nbr[offsets[q] .. offsets[q] + counts[q]) (the fused single-scale driver).
+  // fuse_votes: lrf[9q + 0..5] holds the RAW eigenvectors (x, z) from lrf_eigen_kernel; the sign votes of
+  // shot.py:40-45 run here (the second pass over the same neighbours then hits L1) and the final frame is written
+  // back to lrf[9q + 0..8].
+  // worklist != nullptr: only the queries worklist[0 .. *work_count) (the ones shot_fast_kernel handed over); otherwise
+  // all nq of them.
+  // nbr_stride = 4: `nbr` is the fused driver's list of 16-byte entries (float32 offset, position | flag << 31), the
+  // position is word 3 of an entry and offsets / counts are in entries; the flag (neighbour at distance 0) is masked:
+  // this kernel decides that in float64 itself. nbr_stride = 1: plain int32 positions.
   __shared__ __align__(16) unsigned long long keys[kKeyCount];
   __shared__ __align__(16) float vals[kValCount];
   __shared__ int part[3][kBlockQueryWarps];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const double inv_radius = 1.0 / radius;
   const int nbr_word = nbr_stride - 1;
-  const int n_items = *work_count;
+  const int n_items = worklist != nullptr ? *work_count : int(nq);
   for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-    const int64_t q = worklist[item];
+    const int64_t q = worklist != nullptr ? worklist[item] : item;
+    // values are gated by their keys: only the keys are cleared (16 bytes per thread and store)
     for (int j = tid; j < kKeyCount / 2; j += kBlockQueryWarps * 32) reinterpret_cast<uint4*>(keys)[j] = make_uint4(0u, 0u, 0u, 0u);
     const double qx = __ldg(queries + 3 * q), qy = __ldg(queries + 3 * q + 1), qz = __ldg(queries + 3 * q + 2);
     const int64_t begin = offsets[q], end = counts ? begin + counts[q] : offsets[q + 1];
@@ -562,7 +394,7 @@ __global__ void __launch_bounds__(kBlockQueryWarps * 32)
       for (int k = 0; k < 9; ++k) f[k] = (k % 4 == 0) ? 1.0 : 0.0;  // shot.py:24-25
       if (tid < 9) lrf[9 * q + tid] = (tid % 4 == 0) ? 1.0 : 0.0;
     } else {
-      double x[3] = {lrf[9 * q], lrf[9 * q + 1], lrf[9 * q + 2]}, z[3] = {lrf[9 * q + 3], lrf[9 * q + 4], lrf[9 * q + 5]};
+      const double x[3] = {lrf[9 * q], lrf[9 * q + 1], lrf[9 * q + 2]}, z[3] = {lrf[9 * q + 3], lrf[9 * q + 4], lrf[9 * q + 5]};
       int neg_x = 0, neg_z = 0;
       for (int64_t i = begin + tid; i < end; i += kBlockQueryWarps * 32) {
         const double4 p = load_pt(g.pts + (__ldg(nbr + i * nbr_stride + nbr_word) & 0x7fffffff));
@@ -578,11 +410,7 @@ __global__ void __launch_bounds__(kBlockQueryWarps * 32)
 #pragma unroll
       for (int w = 0; w < kBlockQueryWarps; ++w) { neg_x += part[0][w]; neg_z += part[1][w]; }
       const int k_all = int(end - begin);
-      if (neg_x > k_all - neg_x) { x[0] = -x[0]; x[1] = -x[1]; x[2] = -x[2]; }
-      if (neg_z > k_all - neg_z) { z[0] = -z[0]; z[1] = -z[1]; z[2] = -z[2]; }
-      const double y[3] = {z[1] * x[2] - z[2] * x[1], z[2] * x[0] - z[0] * x[2], z[0] * x[1] - z[1] * x[0]};
-#pragma unroll
-      for (int a = 0; a < 3; ++a) { f[3 * a] = x[a]; f[3 * a + 1] = y[a]; f[3 * a + 2] = z[a]; }
+      shot_frame(x, z, neg_x > k_all - neg_x, neg_z > k_all - neg_z, f);
       if (tid == 0) {
 #pragma unroll
         for (int k = 0; k < 9; ++k) lrf[9 * q + k] = f[k];
@@ -600,16 +428,10 @@ __global__ void __launch_bounds__(kBlockQueryWarps * 32)
         const double4 p = load_pt(g.pts + s), n = load_pt(g.nrm + s);
         const double cx = p.x - qx, cy = p.y - qy, cz = p.z - qz;
         const double d2 = rdist3(cx, cy, cz);
-        if (d2 > 0.0) {  // shot.py:213
+        if (d2 > 0.0) {  // shot.py:213: neighbours at distance 0 (the query itself, duplicates) are dropped
           active = true;
           ++positive;
-          const double rho = sqrt(d2);
-          const double X = frame_dot(cx, cy, cz, f[0], f[3], f[6]);
-          const double Y = frame_dot(cx, cy, cz, f[1], f[4], f[7]);
-          const double Z = frame_dot(cx, cy, cz, f[2], f[5], f[8]);
-          double cosine = n.x * f[2] + n.y * f[5] + n.z * f[8];
-          cosine = fmin(1.0, fmax(-1.0, cosine));
-          d = shot_decide(X, Y, Z, cosine, rho, radius, inv_radius);
+          d = shot_decide_in_frame(cx, cy, cz, n.x, n.y, n.z, f, sqrt(d2), radius, inv_radius);
           key = shot_order_key(d.key, uint32_t(i - begin));
           atomicMax(keys + kKeyOwn + d.own, key);
           atomicMax(keys + kKeyCos + d.cos_nb, key);
@@ -617,28 +439,18 @@ __global__ void __launch_bounds__(kBlockQueryWarps * 32)
         }
       }
       __syncthreads();
-      if (active) {
-        const bool win_own = keys[kKeyOwn + d.own] == key;
-        const bool win_cos = keys[kKeyCos + d.cos_nb] == key;
-        const bool win_az = keys[kKeyAz + d.az_nb] == key;
-        float a_az = 0.0f;
-        if (win_own || win_az) a_az = shot_azimuth(d);
-        if (win_own) {
-          float own_vol, other_vol;
-          shot_elevation(d, own_vol, other_vol);
-          vals[kValOwn + d.own] = (1.0f - d.a_cos) + d.own_shell + own_vol + (1.0f - a_az);
-          vals[kValRad + d.own] = d.other_shell;
-          vals[kValEl + d.own] = other_vol;
-        }
-        if (win_cos) vals[kValCos + d.cos_nb] = d.a_cos;
-        if (win_az) vals[kValAz + d.az_nb] = a_az;
-      }
+      if (active)
+        shot_store_winner(d, keys[kKeyOwn + d.own] == key, keys[kKeyCos + d.cos_nb] == key, keys[kKeyAz + d.az_nb] == key,
+                          vals);
       __syncthreads();  // the stores above are ordered before the next round's key updates
     }
     positive = warp_sum(positive);
     if (lane == 0) part[2][warp] = positive;
     __syncthreads();
-    if (warp == 0) {  // the warp kernel's assembly, lane for lane
+    if (warp == 0) {
+      // assembly: lane handles the groups {lane, lane + 32, lane + 64} of four consecutive bins (one (cosine, azimuth)
+      // cell: the radial / elevation partners are inside the group) -> eight 16-byte table reads and one 16-byte
+      // store per group
       positive = 0;
 #pragma unroll
       for (int w = 0; w < kBlockQueryWarps; ++w) positive += part[2][w];
@@ -683,9 +495,9 @@ __global__ void __launch_bounds__(kBlockQueryWarps * 32)
 
 // ---- S2, fast path: float32-filtered decisions -----------------------------------------------------------------------
 // One warp per query with at most 128 neighbours (four per lane, kept in registers; a slot's code is skipped when the
-// query has no neighbour for it). Round 1's kernel (above) issues ~1650 warp instructions per query, half of them
-// float64, re-gathers the neighbours for the frame's sign votes and keeps 11 KB of tables per warp (20 warps per SM).
-// Here:
+// query has no neighbour for it). Round 1's float64 kernel, a warp per query, issued ~1650 warp instructions per query,
+// half of them float64, re-gathered the neighbours for the frame's sign votes and kept 11 KB of tables per warp (20
+// warps per SM). Here:
 //   * in the fused driver the neighbour arrives as the float32 image of the EXACT float64 offset p - q that the search
 //     kernel had in registers (16-byte list entries: offset + position), so nothing is gathered but the float32
 //     normal and all margins are relative (8 u rho); caller-provided lists gather the grid's cell-relative float32
@@ -1044,14 +856,12 @@ __global__ void __launch_bounds__(kFastWarpsPerBlock * 32, kMinBlocks)
           if (lane < 9) lrf[9 * q + lane] = (lane % 4 == 0) ? 1.0 : 0.0;
         } else {
           const double* frame = lrf + 9 * q;
-          const double sx = double(fsx), sz = double(fsz);
-          const double x[3] = {sx * frame[0], sx * frame[1], sx * frame[2]}, z[3] = {sz * frame[3], sz * frame[4], sz * frame[5]};
-          const double y[3] = {z[1] * x[2] - z[2] * x[1], z[2] * x[0] - z[0] * x[2], z[0] * x[1] - z[1] * x[0]};
+          double f[9];
+          shot_frame(frame, frame + 3, fsx < 0.0f, fsz < 0.0f, f);
           __syncwarp();
           if (lane < 3) {
-            lrf[9 * q + 3 * lane + 0] = lane == 0 ? x[0] : (lane == 1 ? x[1] : x[2]);
-            lrf[9 * q + 3 * lane + 1] = lane == 0 ? y[0] : (lane == 1 ? y[1] : y[2]);
-            lrf[9 * q + 3 * lane + 2] = lane == 0 ? z[0] : (lane == 1 ? z[1] : z[2]);
+#pragma unroll
+            for (int c = 0; c < 3; ++c) lrf[9 * q + 3 * lane + c] = lane == 0 ? f[c] : (lane == 1 ? f[3 + c] : f[6 + c]);
           }
         }
       }
@@ -1127,7 +937,7 @@ static bool env_flag(const char* name) {
 
 // Descriptors of nq queries: shot_fast_kernel on everything, then the exact kernel on the queries the fast one handed
 // over (more than 128 neighbours, a decision inside its float32 margin, or two competitors float32 cannot order).
-// SF_SHOT_EXACT=1 sends every query to the exact kernel (the tests compare the two).
+// SF_SHOT_EXACT=1 sends every query to the exact kernel (the tests' reference for the fast one).
 //   records == false : `list` = int32 positions of a CSR (offsets[nq + 1]), lrf = the final frames
 //   records == true  : the fused driver's padded list of float4 entries (offsets + counts), lrf = raw eigenvectors,
 //                      frame32 = their float32 images (lrf_eigen_kernel)
@@ -1137,15 +947,8 @@ static int launch_descriptor(sf_grid* g, const double* queries, int64_t nq, doub
                              int write_frame, int min_nb, int normalize, void* out, int out_is_f64, int32_t* worklist,
                              int32_t* work_count, const int32_t* status, cudaStream_t stream,
                              bool work_count_is_reset = false) {
-  const size_t smem = size_t(kShotWarpsPerBlock) * kShotSmemPerWarp;
   SF_REQUIRE(reinterpret_cast<uintptr_t>(out) % 16 == 0, SF_ERR_ARG, "SHOT output rows must be 16-byte aligned");
   SF_REQUIRE(nq < (int64_t(1) << 31), SF_ERR_ARG, "SHOT: %lld queries in one call", (long long)nq);
-  static bool configured = false;
-  if (!configured) {
-    SF_CUDA(cudaFuncSetAttribute(shot_descriptor_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SF_CUDA(cudaFuncSetAttribute(shot_descriptor_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    configured = true;
-  }
   const bool exact_only = env_flag("SF_SHOT_EXACT");
   const int fuse_votes = records ? 1 : 0;
   const GridView view = g->view();
@@ -1166,7 +969,8 @@ static int launch_descriptor(sf_grid* g, const double* queries, int64_t nq, doub
     fp.min_nb = min_nb;
     fp.normalize = normalize;
     if (!work_count_is_reset) SF_CUDA(cudaMemsetAsync(work_count, 0, sizeof(int32_t), stream));
-    // persistent: 148 SMs x resident blocks (7.6 KB of tables + staging per warp), capped by the work
+    // persistent: 148 SMs x 2 resident blocks of 8 warps (7.6 KB of tables + staging per warp), capped by the work
+    // (123 registers; the shapes with more warps per SM spill)
     auto launch = [&](auto kernel, auto* typed_out, int warps, int per_sm) -> cudaError_t {
       const size_t fast_smem = size_t(warps) * kFastWordsPerWarp * 4;
       cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(fast_smem));
@@ -1179,57 +983,30 @@ static int launch_descriptor(sf_grid* g, const double* queries, int64_t nq, doub
                                                         worklist, work_count, status);
       return cudaGetLastError();
     };
-    // SF_FAST_SHAPE = <warps per block><resident blocks per SM> the kernel is compiled for: tuning only
-    //   82: 126 registers, 16 warps per SM;  73: 96 registers, 21 warps;  102: 96 registers, 20 warps;
-    //   63: 112 registers, 18 warps;  83: 80 registers, 24 warps (spills)
-    const char* shape_env = getenv("SF_FAST_SHAPE");
-    const int shape = shape_env != nullptr ? atoi(shape_env) : 82;
     float* fo = static_cast<float*>(out);
     double* dout = static_cast<double*>(out);
     if (out_is_f64) {
       if (records) SF_CUDA(launch(shot_fast_kernel<double, true, 8, 2>, dout, 8, 2));
       else SF_CUDA(launch(shot_fast_kernel<double, false, 8, 2>, dout, 8, 2));
-    } else if (!records) {
-      SF_CUDA(launch(shot_fast_kernel<float, false, 8, 2>, fo, 8, 2));
-    } else if (shape == 73) {
-      SF_CUDA(launch(shot_fast_kernel<float, true, 7, 3>, fo, 7, 3));
-    } else if (shape == 102) {
-      SF_CUDA(launch(shot_fast_kernel<float, true, 10, 2>, fo, 10, 2));
-    } else if (shape == 63) {
-      SF_CUDA(launch(shot_fast_kernel<float, true, 6, 3>, fo, 6, 3));
-    } else if (shape == 83) {
-      SF_CUDA(launch(shot_fast_kernel<float, true, 8, 3>, fo, 8, 3));
     } else {
-      SF_CUDA(launch(shot_fast_kernel<float, true, 8, 2>, fo, 8, 2));
+      if (records) SF_CUDA(launch(shot_fast_kernel<float, true, 8, 2>, fo, 8, 2));
+      else SF_CUDA(launch(shot_fast_kernel<float, false, 8, 2>, fo, 8, 2));
     }
   }
-  // exact kernel, persistent-style: 148 SMs x 3 resident blocks (62 KB shared memory each), capped by the work
-  const int64_t blocks_needed = (nq + kShotWarpsPerBlock - 1) / kShotWarpsPerBlock;
-  const unsigned blocks = unsigned(blocks_needed < 148 * 3 ? blocks_needed : 148 * 3);
+  // the exact kernel, a block per query, on the work list of the fast kernel or on every query (as many blocks as the
+  // device holds at once; each strides over the list, whose length only the device knows)
+  const unsigned blocks = unsigned(std::min<int64_t>(nq, 148 * 8));
   const int32_t* wl = exact_only ? nullptr : worklist;
   const int32_t* nbr = static_cast<const int32_t*>(list);
   const int stride = records ? 4 : 1;
-  if (wl != nullptr && !env_flag("SF_SHOT_WARP_WORKLIST")) {
-    // the work list of the fast kernel: a block per query (as many blocks as the device holds at once; each strides over
-    // the list, whose length only the device knows)
-    const unsigned list_blocks = unsigned(std::min<int64_t>(nq, 148 * 8));
-    if (out_is_f64)
-      shot_descriptor_block_kernel<double><<<list_blocks, kBlockQueryWarps * 32, 0, stream>>>(
-          view, queries, radius, offsets, counts, nbr, lrf, fuse_votes, min_nb, normalize, static_cast<double*>(out), wl,
-          work_count, stride, status);
-    else
-      shot_descriptor_block_kernel<float><<<list_blocks, kBlockQueryWarps * 32, 0, stream>>>(
-          view, queries, radius, offsets, counts, nbr, lrf, fuse_votes, min_nb, normalize, static_cast<float*>(out), wl,
-          work_count, stride, status);
-  } else if (out_is_f64) {
-    shot_descriptor_kernel<double><<<blocks, kShotWarpsPerBlock * 32, smem, stream>>>(
+  if (out_is_f64)
+    shot_descriptor_block_kernel<double><<<blocks, kBlockQueryWarps * 32, 0, stream>>>(
         view, queries, nq, radius, offsets, counts, nbr, lrf, fuse_votes, min_nb, normalize, static_cast<double*>(out), wl,
         work_count, stride, status);
-  } else {
-    shot_descriptor_kernel<float><<<blocks, kShotWarpsPerBlock * 32, smem, stream>>>(
+  else
+    shot_descriptor_block_kernel<float><<<blocks, kBlockQueryWarps * 32, 0, stream>>>(
         view, queries, nq, radius, offsets, counts, nbr, lrf, fuse_votes, min_nb, normalize, static_cast<float*>(out), wl,
         work_count, stride, status);
-  }
   SF_CUDA(cudaGetLastError());
   return SF_OK;
 }

@@ -64,25 +64,20 @@ void hm_lrf(const double* point, const double* nbrs, int k, double radius, doubl
   for (int j = 0; j < 6; ++j) m[j] /= sw;
   double eval[3], evec[3][3];
   eigh3(m, eval, evec);
-  double x[3] = {evec[2][0], evec[2][1], evec[2][2]}, z[3] = {evec[0][0], evec[0][1], evec[0][2]};
+  const double* x = evec[2];
+  const double* z = evec[0];
   int neg_x = 0, neg_z = 0;
   for (int i = 0; i < k; ++i) {
     const double cx = nbrs[3 * i] - point[0], cy = nbrs[3 * i + 1] - point[1], cz = nbrs[3 * i + 2] - point[2];
     neg_x += (cx * x[0] + cy * x[1] + cz * x[2]) < 0.0;
     neg_z += (cx * z[0] + cy * z[1] + cz * z[2]) < 0.0;
   }
-  if (neg_x > k - neg_x) for (int a = 0; a < 3; ++a) x[a] = -x[a];
-  if (neg_z > k - neg_z) for (int a = 0; a < 3; ++a) z[a] = -z[a];
-  const double y[3] = {z[1] * x[2] - z[2] * x[1], z[2] * x[0] - z[0] * x[2], z[0] * x[1] - z[1] * x[0]};
-  for (int a = 0; a < 3; ++a) {
-    lrf9[3 * a + 0] = x[a];
-    lrf9[3 * a + 1] = y[a];
-    lrf9[3 * a + 2] = z[a];
-  }
+  shot_frame(x, z, neg_x > k - neg_x, neg_z > k - neg_z, lrf9);
 }
 
-// Mirrors shot_descriptor_kernel for one query: compact winner tables, neighbours taken 32 at a time (key pass,
-// then value pass), atomicMax replaced by a sequential max.
+// Mirrors shot_descriptor_block_kernel for one query: compact winner tables, neighbours taken 32 at a time (key pass,
+// then value pass; the kernel takes 128, which changes nothing since keys are unique), atomicMax replaced by a
+// sequential max.
 void hm_shot_descriptor(const double* point, const double* nbrs, const double* normals, int k, double radius,
                         const double* f, int normalize, int min_nb, float* out352) {
   std::vector<uint64_t> keys(kKeyCount, 0u);
@@ -102,13 +97,8 @@ void hm_shot_descriptor(const double* point, const double* nbrs, const double* n
       if (!(d2 > 0.0)) continue;
       active[lane] = true;
       ++positive;
-      const double rho = sqrt(d2);
-      const double X = frame_dot(cx, cy, cz, f[0], f[3], f[6]);
-      const double Y = frame_dot(cx, cy, cz, f[1], f[4], f[7]);
-      const double Z = frame_dot(cx, cy, cz, f[2], f[5], f[8]);
-      double cosine = normals[3 * i] * f[2] + normals[3 * i + 1] * f[5] + normals[3 * i + 2] * f[8];
-      cosine = fmin(1.0, fmax(-1.0, cosine));
-      d[lane] = shot_decide(X, Y, Z, cosine, rho, radius, inv_radius);
+      d[lane] = shot_decide_in_frame(cx, cy, cz, normals[3 * i], normals[3 * i + 1], normals[3 * i + 2], f, sqrt(d2),
+                                     radius, inv_radius);
       key[lane] = shot_order_key(d[lane].key, uint32_t(i));
       if (key[lane] > keys[kKeyOwn + d[lane].own]) keys[kKeyOwn + d[lane].own] = key[lane];
       if (key[lane] > keys[kKeyCos + d[lane].cos_nb]) keys[kKeyCos + d[lane].cos_nb] = key[lane];
@@ -117,19 +107,8 @@ void hm_shot_descriptor(const double* point, const double* nbrs, const double* n
     for (int lane = 0; lane < 32; ++lane) {
       if (!active[lane]) continue;
       const ShotDecision& e = d[lane];
-      const bool win_own = keys[kKeyOwn + e.own] == key[lane], win_cos = keys[kKeyCos + e.cos_nb] == key[lane],
-                 win_az = keys[kKeyAz + e.az_nb] == key[lane];
-      float a_az = 0.0f;
-      if (win_own || win_az) a_az = shot_azimuth(e);
-      if (win_own) {
-        float own_vol, other_vol;
-        shot_elevation(e, own_vol, other_vol);
-        vals[kValOwn + e.own] = (1.0f - e.a_cos) + e.own_shell + own_vol + (1.0f - a_az);
-        vals[kValRad + e.own] = e.other_shell;
-        vals[kValEl + e.own] = other_vol;
-      }
-      if (win_cos) vals[kValCos + e.cos_nb] = e.a_cos;
-      if (win_az) vals[kValAz + e.az_nb] = a_az;
+      shot_store_winner(e, keys[kKeyOwn + e.own] == key[lane], keys[kKeyCos + e.cos_nb] == key[lane],
+                        keys[kKeyAz + e.az_nb] == key[lane], vals.data());
     }
   }
   double sq = 0.0;
@@ -329,12 +308,7 @@ int hm_shot_descriptor_fast(const double* point, const double* nbrs, const doubl
     if (neg_x > k - neg_x) fsx = -1.0f;
     if (neg_z > k - neg_z) fsz = -1.0f;
   }
-  if (frame_out9 != nullptr && fuse_votes) {
-    const double sx = fsx, sz = fsz;
-    const double x[3] = {sx * frame[0], sx * frame[1], sx * frame[2]}, z[3] = {sz * frame[3], sz * frame[4], sz * frame[5]};
-    const double y[3] = {z[1] * x[2] - z[2] * x[1], z[2] * x[0] - z[0] * x[2], z[0] * x[1] - z[1] * x[0]};
-    for (int a = 0; a < 3; ++a) { frame_out9[3 * a] = x[a]; frame_out9[3 * a + 1] = y[a]; frame_out9[3 * a + 2] = z[a]; }
-  }
+  if (frame_out9 != nullptr && fuse_votes) shot_frame(frame, frame + 3, fsx < 0.0f, fsz < 0.0f, frame_out9);
   std::vector<ShotFastRecord> rec(k);
   std::vector<char> act(k, 0);
   int positive = 0;

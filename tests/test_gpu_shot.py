@@ -277,10 +277,11 @@ def test_calls_without_host_synchronisation_check_their_assumptions():
     assert np.array_equal(rows(spec, sparse_q + np.array([0.0, 0.0, 0.5])), want_moved) and spec.poll() == 0
 
 
-def test_block_per_query_kernel_equals_the_warp_kernel_on_the_work_list(monkeypatch):
+def test_handed_over_queries_get_the_exact_rows(monkeypatch):
     """The queries the float32 kernel hands over are finished by shot_descriptor_block_kernel (a block per query, four
-    warps sharing the winner tables); SF_SHOT_WARP_WORKLIST=1 sends them to the warp-per-query float64 kernel instead:
-    the same rows bit for bit, frames included — also with more than 128 neighbours per query (everything handed over)."""
+    warps sharing the winner tables), the float64 kernel that SF_SHOT_EXACT=1 runs on every query: a query with more
+    than 128 neighbours (always handed over, and more than one round of the block's 128 threads) gets the exact run's
+    row bit for bit, at least as many rows as were handed over are bit-identical, and the frames are identical."""
     import torch
 
     from shot_fpfh_b200 import ops
@@ -292,17 +293,29 @@ def test_block_per_query_kernel_equals_the_warp_kernel_on_the_work_list(monkeypa
     for spacings, stride in ((5.0, 2), (8.0, 40)):  # K ~ 71: a few hundred handed over; K ~ 190: nearly all of them
         radius = spacings * synthetic.mean_spacing(n)
         q_dev = upload(np.ascontiguousarray(pts[::stride]))
+        nq = q_dev.shape[0]
         grid = Grid().build(p_dev, n_dev, radius)
         got = {}
-        for flag in ("0", "1"):
-            monkeypatch.setenv("SF_SHOT_WARP_WORKLIST", flag)
+        for exact in (False, True):
+            if exact:
+                monkeypatch.setenv("SF_SHOT_EXACT", "1")
             d, lrf, pairs = ops.shot_single_scale(grid, q_dev, radius, 10, True, out_dtype=torch.float32, want_lrf=True,
                                                   want_pairs=True)
             torch.cuda.synchronize()
-            got[flag] = (d.clone(), lrf.clone(), ops.shot_last_deferred())
-        assert got["0"][2] == got["1"][2] and got["0"][2] > (50 if spacings == 5.0 else 0.9 * q_dev.shape[0])
-        assert torch.equal(got["0"][0], got["1"][0]) and torch.equal(got["0"][1], got["1"][1])
-        assert bool((got["0"][0].abs().sum(dim=1) > 0).float().mean() > 0.99)
+            got[exact] = (d.clone(), lrf.clone(), ops.shot_last_deferred(), pairs)
+            monkeypatch.delenv("SF_SHOT_EXACT", raising=False)
+        (rows, frames, deferred, pairs), (rows_e, frames_e, deferred_e, _) = got[False], got[True]
+        offsets = ops.radius_csr(grid, q_dev, radius, count_only=True)[0]
+        k = offsets[1:] - offsets[:-1]
+        assert int(k.sum()) == pairs  # the fused driver found the same neighbourhoods
+        big = k > 128
+        assert deferred > (50 if spacings == 5.0 else 0.9 * nq) and deferred_e == nq
+        if spacings == 8.0:
+            assert bool(big.float().mean() > 0.9)
+        assert torch.equal(rows[big], rows_e[big]) and torch.equal(frames, frames_e)
+        assert int((rows == rows_e).all(dim=1).sum()) >= deferred
+        for r in (rows, rows_e):
+            assert bool((r.abs().sum(dim=1) > 0).float().mean() > 0.99)
         grid.close()
 
 
