@@ -494,8 +494,10 @@ __global__ void __launch_bounds__(kBlockQueryWarps * 32)
 }
 
 // ---- S2, fast path: float32-filtered decisions -----------------------------------------------------------------------
-// One warp per query with at most 128 neighbours (four per lane, kept in registers; a slot's code is skipped when the
-// query has no neighbour for it). Round 1's float64 kernel, a warp per query, issued ~1650 warp instructions per query,
+// One warp per query with at most 128 neighbours (four slots of 32 per lane; a slot's code is skipped when the query
+// has no neighbour for it). Slots 0-2 keep their state in registers; slot 3, which only the 6 % of the C2 queries with
+// more than 96 neighbours use, keeps it in shared memory between the phases: the registers it would hold cost 20 -> 16
+// warps per SM on every query. Round 1's float64 kernel, a warp per query, issued ~1650 warp instructions per query,
 // half of them float64, re-gathered the neighbours for the frame's sign votes and kept 11 KB of tables per warp (20
 // warps per SM). Here:
 //   * in the fused driver the neighbour arrives as the float32 image of the EXACT float64 offset p - q that the search
@@ -513,6 +515,7 @@ __global__ void __launch_bounds__(kBlockQueryWarps * 32)
 // of one of its neighbours sits inside its float32 margin, or when two neighbours that compete for a bin are closer
 // in distance than float32 can order (`amb_margin`).
 constexpr int kFastSlots = 4;
+constexpr int kFastRegSlots = 3;  // slots whose state stays in registers from the decisions to the value phases
 constexpr int kFastMaxK = 32 * kFastSlots;
 constexpr int kFastTableWords = kKeyCount + kShotLen;  // three key tables + the output bins
 constexpr int kFrame32Stride = 12;                          // floats per query of lrf_eigen_kernel's float32 frame (x, y, z, pad)
@@ -521,6 +524,12 @@ constexpr int kFrame32Stride = 12;                          // floats per query 
 constexpr int kFastWordsPerWarp = kFastTableWords + 4 + 2 * (kFastMaxK * 4 + kFrame32Stride + 4);
 constexpr float kFastN2 = 1.001f;                        // unit normals up to rounding
 static_assert(kFastMaxK <= (1 << kFastIndexBits), "a neighbour's list position must fit the key's index bits");
+// The per-lane record of the last slot: its three addresses, its key and its five values, word f of lane l at word
+// 32 f + l of the staging buffer the query's entries came from (read into registers before the record is written;
+// the TMA unit refills that buffer only for the query after the next).
+enum { kRecAddr = 0, kRecKey = 3, kRecOwn, kRecCos, kRecAz, kRecRad, kRecEl, kRecWords };
+static_assert(kFastSlots == kFastRegSlots + 1, "one slot outside the registers");
+static_assert(kRecWords * 32 <= kFastRegSlots * 32 * 4, "the record overlays the entries of the register slots only");
 
 struct FastParams {
   float radius, inv_radius, edge32;
@@ -544,6 +553,9 @@ __device__ __forceinline__ float smem_ld_f32(uint32_t addr) {
 }
 __device__ __forceinline__ void smem_st_f32(uint32_t addr, float v) {
   asm volatile("st.shared.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
+}
+__device__ __forceinline__ void smem_st_u32(uint32_t addr, uint32_t v) {
+  asm volatile("st.shared.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
 }
 __device__ __forceinline__ void smem_red_max(uint32_t addr, uint32_t v) {
   asm volatile("red.shared.max.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
@@ -570,8 +582,8 @@ __global__ void __launch_bounds__(kFastWarpsPerBlock * 32, kMinBlocks)
   constexpr int kGroups = kShotLen / 4, kGroupRounds = (kGroups + 31) / 32;
   const uint32_t amb_span = (fp.amb_margin << kFastIndexBits) | ((1u << kFastIndexBits) - 1u);
 
-  // Software pipeline over the warp's queries, two deep: at the top of an iteration the header (list position,
-  // neighbour count) of the query after the next is requested, and one lane asks the TMA unit for the NEXT query's list
+  // Software pipeline over the warp's queries, two deep: in an iteration the header (list position, neighbour count)
+  // of the query after the next is requested, and at its top one lane asks the TMA unit for the NEXT query's list
   // entries and frame (two bulk copies into one of the warp's two staging buffers, completion on that buffer's
   // mbarrier): a whole iteration hides the copy (the 117 MB list comes from DRAM), and no register is carried for it.
   constexpr int kStageBytes = kFastMaxK * 16 + kFrame32Stride * 4 + 16;  // entries, frame, mbarrier (+ padding)
@@ -618,13 +630,16 @@ __global__ void __launch_bounds__(kFastWarpsPerBlock * 32, kMinBlocks)
   for (; q < nq;) {
     const int64_t q_next = q + warps_total;
     stage(q_next, begin_next, K_next, buffer ^ 1);  // (its header was requested an iteration ago)
-    int64_t begin_after;
-    int K_after;
-    header(q_next + warps_total, begin_after, K_after);
     bool defer = K > kFastMaxK;  // too many for four per lane: the exact kernel takes it
     const bool work = K > 0 && !defer;
-    uint32_t addr[kFastSlots][3], key[kFastSlots];
-    float v_own[kFastSlots], v_cos[kFastSlots], v_az[kFastSlots], v_rad[kFastSlots], v_el[kFastSlots];
+    uint32_t addr[kFastRegSlots][3], key[kFastRegSlots];
+    float v_own[kFastRegSlots], v_cos[kFastRegSlots], v_az[kFastRegSlots], v_rad[kFastRegSlots], v_el[kFastRegSlots];
+    // the last slot's record (warp-uniform: only when K > 96)
+    const bool last_slot = K > kFastRegSlots * 32;
+    const uint32_t rec = stage_base + buffer * kStageBytes + 4u * lane;
+    auto rec_ld = [&](int f) { return smem_ld_u32(rec + 128u * f); };
+    auto rec_ldf = [&](int f) { return smem_ld_f32(rec + 128u * f); };
+    auto rec_st = [&](int f, uint32_t v) { smem_st_u32(rec + 128u * f, v); };
     float fsx = 1.0f, fsz = 1.0f;
     int positive = 0;
     if (work) {
@@ -736,97 +751,143 @@ __global__ void __launch_bounds__(kFastWarpsPerBlock * 32, kMinBlocks)
       // ---- decisions; one fire-and-forget shared max per (neighbour, statement group) ----
       // Per neighbour: the shared-memory byte addresses of its three key slots, its key and its five values. The
       // bins sit kKeyCount words above the key tables: a value goes to (slot of group t) + (kKeyCount - 352 t) words.
+      auto decide = [&](int s, uint32_t(&a)[3], uint32_t& k) {
+        const bool on = (act >> s) & 1u;
+        const float nv[3] = {pb[s].x, pb[s].y, pb[s].z};
+        const float inv_rho = sf_rsqrtf(fmaxf(R2[s], 1e-37f)), rho = R2[s] * inv_rho;
+        ShotFastMargins m;
+        m.e_loc = kRecords ? fp.e_rel * rho : fp.e_abs;
+        m.e_rho = m.e_loc;
+        m.w_rho_min = kRecords ? 0.0f : fp.w_min;
+        m.w_xy_min = kRecords ? 0.01f * rho : fp.w_min;
+        m.n2 = kFastN2;
+        ShotDecision d;
+        // (the cosine margin assumes |n|^2 <= kFastN2: longer normals are left to the exact kernel)
+        const bool sure = shot_decide_fast(fsx * X0[s], fsx * fsz * Y0[s], fsz * Z0[s], fsz * dot3f(nv, az), rho, inv_rho,
+                                           fp.radius, fp.inv_radius, m, d) &&
+                          dot3f(nv, nv) <= kFastN2;
+        unsure = unsure || (on && !sure);
+        const bool use = on && sure;
+        const ShotFastRecord r = shot_fast_record(d, uint32_t(s * 32 + lane));
+        k = use ? r.key : 0u;
+        // (an unsure decision may hold any bin: its addresses are never formed)
+        a[0] = use ? keys_addr + 4u * uint32_t(kKeyOwn + d.own) : trash;
+        a[1] = use ? keys_addr + 4u * uint32_t(kKeyCos + d.cos_nb) : trash;
+        a[2] = use ? keys_addr + 4u * uint32_t(kKeyAz + d.az_nb) : trash;
 #pragma unroll
-      for (int s = 0; s < kFastSlots; ++s) {
+        for (int t = 0; t < 3; ++t) smem_red_max(a[t], k);  // (0 on the trash word: no effect)
+        positive += __popc(__ballot_sync(kFull, on));
+        return r;
+      };
+      // the last slot first: decided after the others, it needs four registers more than there are at 20 warps per SM
+      // (the keys do not depend on the order of the maxima)
+      if (last_slot) {  // (every lane has read the staged entries: the __syncwarp above)
+        uint32_t a[3], k;
+        const ShotFastRecord r = decide(kFastRegSlots, a, k);
+#pragma unroll
+        for (int t = 0; t < 3; ++t) rec_st(kRecAddr + t, a[t]);
+        rec_st(kRecKey, k);
+        rec_st(kRecOwn, __float_as_uint(r.v_own));
+        rec_st(kRecCos, __float_as_uint(r.v_cos));
+        rec_st(kRecAz, __float_as_uint(r.v_az));
+        rec_st(kRecRad, __float_as_uint(r.v_rad));
+        rec_st(kRecEl, __float_as_uint(r.v_el));
+      }
+#pragma unroll
+      for (int s = 0; s < kFastRegSlots; ++s) {
         if (s * 32 < K) {
-          const bool on = (act >> s) & 1u;
-          const float nv[3] = {pb[s].x, pb[s].y, pb[s].z};
-          const float inv_rho = sf_rsqrtf(fmaxf(R2[s], 1e-37f)), rho = R2[s] * inv_rho;
-          ShotFastMargins m;
-          m.e_loc = kRecords ? fp.e_rel * rho : fp.e_abs;
-          m.e_rho = m.e_loc;
-          m.w_rho_min = kRecords ? 0.0f : fp.w_min;
-          m.w_xy_min = kRecords ? 0.01f * rho : fp.w_min;
-          m.n2 = kFastN2;
-          ShotDecision d;
-          // (the cosine margin assumes |n|^2 <= kFastN2: longer normals are left to the exact kernel)
-          const bool sure = shot_decide_fast(fsx * X0[s], fsx * fsz * Y0[s], fsz * Z0[s], fsz * dot3f(nv, az), rho, inv_rho,
-                                             fp.radius, fp.inv_radius, m, d) &&
-                            dot3f(nv, nv) <= kFastN2;
-          unsure = unsure || (on && !sure);
-          const bool use = on && sure;
-          const ShotFastRecord r = shot_fast_record(d, uint32_t(s * 32 + lane));
-          key[s] = use ? r.key : 0u;
+          const ShotFastRecord r = decide(s, addr[s], key[s]);
           v_own[s] = r.v_own; v_cos[s] = r.v_cos; v_az[s] = r.v_az; v_rad[s] = r.v_rad; v_el[s] = r.v_el;
-          // (an unsure decision may hold any bin: its addresses are never formed)
-          addr[s][0] = use ? keys_addr + 4u * uint32_t(kKeyOwn + d.own) : trash;
-          addr[s][1] = use ? keys_addr + 4u * uint32_t(kKeyCos + d.cos_nb) : trash;
-          addr[s][2] = use ? keys_addr + 4u * uint32_t(kKeyAz + d.az_nb) : trash;
-#pragma unroll
-          for (int t = 0; t < 3; ++t) smem_red_max(addr[s][t], key[s]);  // (0 on the trash word: no effect)
-          positive += __popc(__ballot_sync(kFull, on));
         }
       }
       __syncwarp();  // the shared maxima are ordered before the reads below
       defer = __any_sync(kFull, unsure);
     }
+    // the header of the query after the next (requested here rather than at the top: the decisions above need the
+    // registers more, and the rest of the iteration still hides the load)
+    int64_t begin_after;
+    int K_after;
+    header(q_next + warps_total, begin_after, K_after);
     if (work && !defer) {
       // ---- winners (keys are unique: equality = THE winner) and competitors float32 cannot order ----
       // A slot that did not win (or holds no neighbour) is redirected to the warp's trash word, so that the value
       // phases below run without branches: every lane does load - add - store, losers on the trash word.
+      // The last slot re-reads its state from the record in every phase (a bin has one writer per sub-phase, so where
+      // in a sub-phase that slot's load - add - store runs does not change any sum).
       uint32_t closest = 0xffffffffu;  // smallest (winner key - own key - 1) over this lane's losing slots
+      auto winner = [&](uint32_t(&a)[3], uint32_t k) {
+        uint32_t seen[3];
 #pragma unroll
-      for (int s = 0; s < kFastSlots; ++s) {
-        if (s * 32 < K) {
-          uint32_t seen[3];
+        for (int t = 0; t < 3; ++t) seen[t] = smem_ld_u32(a[t]);  // >= k (trash: 0xffffffff; no key is 0)
 #pragma unroll
-          for (int t = 0; t < 3; ++t) seen[t] = smem_ld_u32(addr[s][t]);  // >= key[s] (trash: 0xffffffff; no key is 0)
-#pragma unroll
-          for (int t = 0; t < 3; ++t) {
-            closest = min(closest, seen[t] - key[s] - 1u);  // (a winner wraps to 0xffffffff)
-            addr[s][t] = seen[t] == key[s] ? addr[s][t] + uint32_t(kKeyCount - t * kShotLen) * 4u : trash;
-          }
+        for (int t = 0; t < 3; ++t) {
+          closest = min(closest, seen[t] - k - 1u);  // (a winner wraps to 0xffffffff)
+          a[t] = seen[t] == k ? a[t] + uint32_t(kKeyCount - t * kShotLen) * 4u : trash;
         }
+      };
+#pragma unroll
+      for (int s = 0; s < kFastRegSlots; ++s)
+        if (s * 32 < K) winner(addr[s], key[s]);
+      if (last_slot) {
+        uint32_t a[3] = {rec_ld(kRecAddr), rec_ld(kRecAddr + 1), rec_ld(kRecAddr + 2)};
+        winner(a, rec_ld(kRecKey));
+#pragma unroll
+        for (int t = 0; t < 3; ++t) rec_st(kRecAddr + t, a[t]);
       }
       bool amb = closest < amb_span;  // a winner at most amb_span above one of this lane's keys: unordered
       // ---- values, one writer per bin and sub-phase (loads of a sub-phase first, then its stores) ----
 #pragma unroll
-      for (int s = 0; s < kFastSlots; ++s)
+      for (int s = 0; s < kFastRegSlots; ++s)
         if (s * 32 < K) smem_st_f32(addr[s][0], v_own[s]);  // statements 2 + 5 + 8 + 10
+      if (last_slot) smem_st_f32(rec_ld(kRecAddr), rec_ldf(kRecOwn));
       __syncwarp();
 #pragma unroll
       for (int t = 0; t < 2; ++t) {  // radial partner (statement 3 or 4), then elevation partner (6 or 7)
-        uint32_t dst[kFastSlots], pk[kFastSlots];
-        float cur[kFastSlots];
+        // the own-bin winner's partner bin: its value slot is the own value slot's address with bit 2 (3) flipped,
+        // its own-group key sits kKeyCount words below
+        auto partner = [&](uint32_t own) { return own != trash ? own ^ (4u << t) : trash; };
+        auto partner_key = [&](uint32_t dst) { return smem_ld_u32(dst != trash ? dst - uint32_t(kKeyCount) * 4u : trash); };
+        auto settle = [&](uint32_t dst, uint32_t pk, uint32_t k) {
+          amb = amb || (dst != trash && max(pk, k) - min(pk, k) <= amb_span);
+          return k > pk ? dst : trash;  // (pk of a non-winner: the trash word, above every key)
+        };
+        uint32_t dst[kFastRegSlots], pk[kFastRegSlots];
+        float cur[kFastRegSlots];
 #pragma unroll
-        for (int s = 0; s < kFastSlots; ++s)
+        for (int s = 0; s < kFastRegSlots; ++s)
           if (s * 32 < K) {
-            // the own-bin winner's partner bin: its value slot is the own value slot's address with bit 2 (3) flipped,
-            // its own-group key sits kKeyCount words below
-            dst[s] = addr[s][0] != trash ? addr[s][0] ^ (4u << t) : trash;
-            pk[s] = smem_ld_u32(dst[s] != trash ? dst[s] - uint32_t(kKeyCount) * 4u : trash);
+            dst[s] = partner(addr[s][0]);
+            pk[s] = partner_key(dst[s]);
           }
 #pragma unroll
-        for (int s = 0; s < kFastSlots; ++s)
+        for (int s = 0; s < kFastRegSlots; ++s)
           if (s * 32 < K) {
-            amb = amb || (dst[s] != trash && max(pk[s], key[s]) - min(pk[s], key[s]) <= amb_span);
-            dst[s] = key[s] > pk[s] ? dst[s] : trash;  // (pk of a non-winner: the trash word, above every key)
+            dst[s] = settle(dst[s], pk[s], key[s]);
             cur[s] = smem_ld_f32(dst[s]);
           }
 #pragma unroll
-        for (int s = 0; s < kFastSlots; ++s)
+        for (int s = 0; s < kFastRegSlots; ++s)
           if (s * 32 < K) smem_st_f32(dst[s], cur[s] + (t == 0 ? v_rad[s] : v_el[s]));
+        if (last_slot) {
+          const uint32_t d = partner(rec_ld(kRecAddr));
+          const uint32_t w = settle(d, partner_key(d), rec_ld(kRecKey));
+          smem_st_f32(w, smem_ld_f32(w) + rec_ldf(t == 0 ? kRecRad : kRecEl));
+        }
         __syncwarp();
       }
 #pragma unroll
       for (int t = 1; t < 3; ++t) {  // statement 1, then statement 9
-        float cur[kFastSlots];
+        float cur[kFastRegSlots];
 #pragma unroll
-        for (int s = 0; s < kFastSlots; ++s)
+        for (int s = 0; s < kFastRegSlots; ++s)
           if (s * 32 < K) cur[s] = smem_ld_f32(addr[s][t]);
 #pragma unroll
-        for (int s = 0; s < kFastSlots; ++s)
+        for (int s = 0; s < kFastRegSlots; ++s)
           if (s * 32 < K) smem_st_f32(addr[s][t], cur[s] + (t == 1 ? v_cos[s] : v_az[s]));
+        if (last_slot) {
+          const uint32_t a = rec_ld(kRecAddr + t);
+          smem_st_f32(a, smem_ld_f32(a) + rec_ldf(t == 1 ? kRecCos : kRecAz));
+        }
         __syncwarp();
       }
       defer = __any_sync(kFull, amb);  // float32 cannot order two competitors: the exact kernel redoes the query
@@ -866,6 +927,8 @@ __global__ void __launch_bounds__(kFastWarpsPerBlock * 32, kMinBlocks)
         }
       }
     }
+    // the record's stores and loads are ordered before the TMA unit refills its buffer
+    if (kRecords && last_slot) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     __syncwarp();  // all lanes have read the tables before the next query clears them
     q = q_next;
     begin = begin_next;
@@ -969,8 +1032,9 @@ static int launch_descriptor(sf_grid* g, const double* queries, int64_t nq, doub
     fp.min_nb = min_nb;
     fp.normalize = normalize;
     if (!work_count_is_reset) SF_CUDA(cudaMemsetAsync(work_count, 0, sizeof(int32_t), stream));
-    // persistent: 148 SMs x 2 resident blocks of 8 warps (7.6 KB of tables + staging per warp), capped by the work
-    // (123 registers; the shapes with more warps per SM spill)
+    // persistent: 148 SMs x 2 resident blocks, capped by the work. The fused driver's lists: blocks of 10 warps, 20 per
+    // SM (96 registers without spills; 9.6 KB of tables + staging per warp, 195 KB per SM with the per-block reserve).
+    // Caller-provided lists: blocks of 8 warps (128 registers; at 96 that instantiation spills).
     auto launch = [&](auto kernel, auto* typed_out, int warps, int per_sm) -> cudaError_t {
       const size_t fast_smem = size_t(warps) * kFastWordsPerWarp * 4;
       cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(fast_smem));
@@ -986,10 +1050,10 @@ static int launch_descriptor(sf_grid* g, const double* queries, int64_t nq, doub
     float* fo = static_cast<float*>(out);
     double* dout = static_cast<double*>(out);
     if (out_is_f64) {
-      if (records) SF_CUDA(launch(shot_fast_kernel<double, true, 8, 2>, dout, 8, 2));
+      if (records) SF_CUDA(launch(shot_fast_kernel<double, true, 10, 2>, dout, 10, 2));
       else SF_CUDA(launch(shot_fast_kernel<double, false, 8, 2>, dout, 8, 2));
     } else {
-      if (records) SF_CUDA(launch(shot_fast_kernel<float, true, 8, 2>, fo, 8, 2));
+      if (records) SF_CUDA(launch(shot_fast_kernel<float, true, 10, 2>, fo, 10, 2));
       else SF_CUDA(launch(shot_fast_kernel<float, false, 8, 2>, fo, 8, 2));
     }
   }
