@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SF_ABI_VERSION 12
+#define SF_ABI_VERSION 13
 
 #define SF_OK 0
 #define SF_ERR_CUDA 1     /* a CUDA runtime call or kernel launch failed */
@@ -144,6 +144,25 @@ int sf_iss_saliency(sf_grid* grid, double salient_radius, int32_t min_neighbors,
  * (the count is a host result); *count_host = 0 for an empty handle. */
 int sf_iss_select(sf_grid* grid, const double* saliency_dev, double non_max_radius, int32_t min_neighbors,
                   int32_t* keypoints_dev, int64_t* count_host, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------
+ * O — consistent normal orientation (no counterpart in the reference). Hoppe et al. 1992: signs propagated along the
+ * minimum spanning forest of the k-NN graph; oracle/orientation_oracle.py is the specification. Every entry j != i of
+ * point i's list is an undirected edge {i, j} (found from both ends, it is one edge) with
+ * d = (n_i.x*n_j.x + n_i.y*n_j.y) + n_i.z*n_j.z (float64, no FMA), weight 1 - |d|, flip bit d < 0, and the unique key
+ * (weight, min(i, j), max(i, j)). A point's sign relative to another point of its tree is the XOR of the flip bits on
+ * the tree path between them. In each tree the member with the lowest index keeps its input sign; with towards_host
+ * (3 float64, a viewpoint t) each tree instead takes the sign under which more of its members have n . (t - p) > 0
+ * than < 0 (ties: the lowest-index rule).
+ * ---------------------------------------------------------------------------------------------------------- */
+/* xyz_dev, normals_dev: float64 (n,3); nbr_index_dev: int32 (n, k_stride) ORIGINAL point indices (the lists of
+ * sf_knn with k + 1: self entries are skipped, an index outside [0, n) is an error); towards_host may be NULL.
+ * out_dev: float64 (n,3), the input normals with some negated (may not alias normals_dev). *n_trees_host = number of
+ * trees of the forest. Borůvka rounds with parity labels on the device; synchronises `stream` once per round and once
+ * per pointer-jumping step (O(log n) rounds). */
+int sf_orient_normals(const double* xyz_dev, const double* normals_dev, int64_t n, const int32_t* nbr_index_dev,
+                      int32_t k_stride, const double* towards_host, double* out_dev, int64_t* n_trees_host,
+                      void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * S — SHOT.

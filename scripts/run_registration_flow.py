@@ -4,10 +4,14 @@ compute_descriptors, find_descriptors_matches, run_ransac, run_icp) through THIS
 NumPy arrays in and out at every stage, on a synthetic rigid pair (SURVEY.md 8d generator). BASELINE.json configs[4]
 names a 10M-point pair; the size is an argument:
 
-    python scripts/run_registration_flow.py [n_points] [fpfh] [voxel|iss]
+    python scripts/run_registration_flow.py [n_points] [fpfh] [voxel|iss] [pca|pca_raw]
 
 The keypoint selector is `voxel` (select_keypoints_subsampling, 3.75 spacings: the default) or `iss`
 (select_keypoints_iss, salient radius 5 spacings, non-max radius 3.75 spacings: far fewer keypoints, on salient points).
+The normals are the synthetic surface's analytic ones (the default), or `pca`: compute_normals(k=30) of each cloud,
+oriented by orient_normals (k = 10) towards the cloud's centroid and then negated, so that both clouds' normals point
+away from it, as the analytic ones do. `pca_raw` keeps compute_normals' signs (LAPACK's, a coin flip per point): it
+measures what sign noise does to matching.
 Prints wall-clock per stage and the error of the recovered transform against the known one. (`/root/reference` is not
 on the GPU box, so its `RegistrationPipeline` object cannot be run there; `dropin.install()` binds exactly these
 callables into it.)
@@ -24,13 +28,19 @@ import torch  # noqa: E402
 
 from shot_fpfh_b200 import synthetic  # noqa: E402
 from shot_fpfh_b200.core import RigidTransform  # noqa: E402
-from shot_fpfh_b200.descriptors import ShotMultiprocessor, compute_fpfh_descriptor  # noqa: E402
+from shot_fpfh_b200.descriptors import (  # noqa: E402
+    ShotMultiprocessor,
+    compute_fpfh_descriptor,
+    compute_normals,
+    orient_normals,
+)
 from shot_fpfh_b200.icp import icp_point_to_plane  # noqa: E402
 from shot_fpfh_b200.keypoint_selection import select_keypoints_iss, select_keypoints_subsampling  # noqa: E402
 from shot_fpfh_b200.matching import match_descriptors, ransac_on_matches  # noqa: E402
 
 
-def run(n: int, with_fpfh: bool = False, verbose: bool = True, keypoints: str = "voxel") -> dict:
+def run(n: int, with_fpfh: bool = False, verbose: bool = True, keypoints: str = "voxel",
+        normals_from: str = "analytic") -> dict:
     times = {}
 
     def stage(name, fn):
@@ -49,7 +59,16 @@ def run(n: int, with_fpfh: bool = False, verbose: bool = True, keypoints: str = 
     s = synthetic.mean_spacing(n)
     radius = 5.0 * s
     if verbose:
-        print(f"pair of {n} points, radius {radius:.5f}")
+        print(f"pair of {n} points, radius {radius:.5f}, {normals_from} normals")
+    if normals_from in ("pca", "pca_raw"):
+        def pca(cloud):
+            nrm = compute_normals(cloud, cloud, k=30)
+            return nrm if normals_from == "pca_raw" else -orient_normals(cloud, nrm, k=10, towards=cloud.mean(axis=0))
+
+        normals = stage(f"normals {normals_from} (scan)", lambda: pca(scan))
+        ref_normals = stage(f"normals {normals_from} (ref)", lambda: pca(ref))
+    elif normals_from != "analytic":
+        raise ValueError(f"unknown normals {normals_from!r} (analytic, pca or pca_raw)")
     if keypoints == "iss":
         select = lambda cloud: select_keypoints_iss(cloud, 5.0 * s, 3.75 * s)  # noqa: E731
     elif keypoints == "voxel":
@@ -80,7 +99,7 @@ def run(n: int, with_fpfh: bool = False, verbose: bool = True, keypoints: str = 
         scan, ref, ref_normals, RigidTransform(coarse.rotation, coarse.translation), d_max=2 * s, voxel_size=3.75 * s,
         max_iter=20, rms_threshold=1e-9))
     out = {
-        "n_points": n, "keypoint_selector": keypoints, "keypoints": (int(scan_kp.shape[0]), int(ref_kp.shape[0])), "matches": int(matches[0].shape[0]),
+        "n_points": n, "keypoint_selector": keypoints, "normals": normals_from, "keypoints": (int(scan_kp.shape[0]), int(ref_kp.shape[0])), "matches": int(matches[0].shape[0]),
         "ransac_inlier_ratio": float(ratio),
         "coarse_rotation_error": float(np.abs(coarse.rotation - rot).max()),
         "fine_rotation_error": float(np.abs(fine.rotation - rot).max()),
@@ -96,4 +115,5 @@ def run(n: int, with_fpfh: bool = False, verbose: bool = True, keypoints: str = 
 if __name__ == "__main__":
     size = int(sys.argv[1]) if len(sys.argv) > 1 else 10_000_000
     words = sys.argv[2:]
-    run(size, with_fpfh="fpfh" in words, keypoints="iss" if "iss" in words else "voxel")
+    normals_from = "pca" if "pca" in words else ("pca_raw" if "pca_raw" in words else "analytic")
+    run(size, with_fpfh="fpfh" in words, keypoints="iss" if "iss" in words else "voxel", normals_from=normals_from)

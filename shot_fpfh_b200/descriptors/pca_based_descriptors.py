@@ -5,6 +5,7 @@ smallest eigenvalue of each neighbourhood's covariance (csrc/normals.cu, LAPACK-
 of a normal that is NOT re-oriented by `pre_computed_normals` is the one np.linalg.eigh gives).
 
 This is a "next" row (SURVEY.md §8f #2): it runs upstream of the hot path, in `get_data` (helpers/io_ply.py:259-301).
+`orient_normals` (no counterpart in the reference) gives those normals consistent signs (csrc/orient.cu).
 The other functions of the reference module (sphericity, linearity ... features and their plots) are not on any path
 the pipeline takes and are not provided.
 """
@@ -16,7 +17,7 @@ import numpy.typing as npt
 import torch
 
 from .. import ops
-from ..device import Grid, download, upload
+from ..device import Grid, download, require_cuda, upload
 
 
 def _calibrate_reach(grid_points: torch.Tensor, queries: torch.Tensor, k: int) -> float:
@@ -98,3 +99,41 @@ def compute_normals(
         grid.close()
         normals = ops.pca_normals(pts, int(q.shape[0]), nbr, offsets=offsets, pre_normals=pre)
     return download(normals)
+
+
+def orient_normals(
+    points: npt.NDArray[np.float64],
+    normals: npt.NDArray[np.float64],
+    k: int = 10,
+    towards: npt.ArrayLike | None = None,
+) -> npt.NDArray[np.float64]:
+    """
+    Consistently oriented normals (Hoppe et al. 1992; Open3D's `orient_normals_consistent_tangent_plane`): the signs
+    of `normals` (e.g. `compute_normals` output, whose signs are LAPACK's) are propagated along the minimum spanning
+    forest of the k-nearest-neighbour graph, with edge weight 1 - |n_i . n_j|. Returns a new (n, 3) float64 array: the
+    input normals with some of them negated.
+    Each tree of the forest (one per connected piece of the graph) gets one sign: by default its member with the
+    lowest index keeps its input sign; with `towards` = (x, y, z), a viewpoint, the tree takes the sign under which
+    more of its members have n . (towards - p) > 0 than < 0 (a tie keeps the default).
+    No counterpart in the reference; oracle/orientation_oracle.py states the same computation in NumPy.
+    """
+    require_cuda()
+    pts_h = np.asarray(points, dtype=np.float64).reshape(-1, 3)
+    nrm_h = np.asarray(normals, dtype=np.float64).reshape(-1, 3)
+    if pts_h.shape != nrm_h.shape:
+        raise ValueError(f"points {pts_h.shape} and normals {nrm_h.shape} differ in shape")
+    if not (np.isfinite(pts_h).all() and np.isfinite(nrm_h).all()):
+        raise ValueError("orient_normals: points and normals must be finite")
+    if towards is not None:
+        towards = np.asarray(towards, dtype=np.float64).reshape(3)
+        if not np.isfinite(towards).all():
+            raise ValueError("orient_normals: towards must be finite")
+    n, k = pts_h.shape[0], int(k)
+    if n == 0:
+        return np.empty((0, 3), dtype=np.float64)
+    if k < 1:
+        raise ValueError(f"Expected n_neighbors > 0. Got {k}")
+    pts, nrm = upload(pts_h), upload(nrm_h)
+    nbr = knn_device(pts, pts, k + 1)  # raises for k >= n; the point itself is among its k + 1 nearest
+    out, _ = ops.orient_normals(pts, nrm, nbr, towards)
+    return download(out)

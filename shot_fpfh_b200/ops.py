@@ -112,6 +112,20 @@ def pca_normals(xyz: torch.Tensor, nq: int, nbr_index: torch.Tensor, offsets: to
     return out
 
 
+def orient_normals(xyz: torch.Tensor, normals: torch.Tensor, nbr_index: torch.Tensor,
+                   towards=None) -> tuple[torch.Tensor, int]:
+    """Consistently oriented `normals` (sf_orient_normals) from the (n, K) neighbour lists `nbr_index` (ORIGINAL
+    indices, int32) -> (oriented normals float64 (n, 3), number of trees of the spanning forest)."""
+    n = int(xyz.shape[0])
+    out = torch.empty((n, 3), dtype=torch.float64, device=xyz.device)
+    trees = ctypes.c_int64(0)
+    t = None if towards is None else np.ascontiguousarray(towards, dtype=np.float64).reshape(3)
+    check(lib.sf_orient_normals(ptr(xyz), ptr(normals), n, ptr(nbr_index), int(nbr_index.shape[1]) if n else 1,
+                                None if t is None else t.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), ptr(out),
+                                ctypes.byref(trees), stream_ptr()))
+    return out, int(trees.value)
+
+
 def iss_saliency(grid: Grid, salient_radius: float, min_neighbors: int, gamma_21: float, gamma_32: float,
                  want_counts: bool = False, want_eigvals: bool = False):
     """
