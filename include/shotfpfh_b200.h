@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SF_ABI_VERSION 13
+#define SF_ABI_VERSION 14
 
 #define SF_OK 0
 #define SF_ERR_CUDA 1     /* a CUDA runtime call or kernel launch failed */
@@ -70,11 +70,17 @@ int sf_grid_geometry(const double* lo3, const double* hi3, double radius, double
  * sizes its neighbour list from its last synchronising call on this cloud instead of reading the size back. Both assumptions are CHECKED ON THE DEVICE: when one
  * fails the kernels of these calls do nothing, and sf_grid_poll — to be called after synchronising the stream, before
  * the results are used — reports a non-zero status (1: a point outside the assumed box, 2: neighbour list too small)
- * and returns the handle to synchronising calls; the caller then simply repeats its calls. */
+ * and returns the handle to synchronising calls; the caller then simply repeats its calls. The calls copy nothing
+ * back: sf_grid_poll reads the device-side flag itself (a synchronous 4-byte copy). */
 int sf_grid_set_speculative(sf_grid* grid, int32_t mode);
 int sf_grid_poll(sf_grid* grid, int32_t* status);
 /* Copies perm[n] (cell-sorted position -> original index) and/or its inverse into caller buffers (NULL = skip). */
 int sf_grid_permutation(const sf_grid* grid, int32_t* perm_out_dev, int32_t* inv_perm_out_dev, void* stream);
+/* Copies the grid's cell-sorted arrays into caller buffers (NULL = skip): pts (n,4) float64 (xyz, original index as
+ * int64 bits), nrm (n,4) float64, xyzc (n,4) float32 (cell-relative xyz, cell bits), nrm32 (n,4) float32 and
+ * cell_start[ncells + 1] int32. nrm / nrm32 only for a grid built with normals. */
+int sf_grid_arrays(const sf_grid* grid, double* pts_out_dev, double* nrm_out_dev, float* xyzc_out_dev,
+                   float* nrm32_out_dev, int32_t* cell_start_out_dev, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * G — fixed-radius search.  Replaces `KDTree.query_radius(X, r[, return_distance=True])`

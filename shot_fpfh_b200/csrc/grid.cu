@@ -285,7 +285,6 @@ static void free_all(sf_grid* g) {
   cudaFree(g->cell_start); cudaFree(g->cell_count); cudaFree(g->keys_in); cudaFree(g->keys_out);
   cudaFree(g->vals_in); cudaFree(g->bbox); cudaFree(g->cub_temp);
   cudaFree(g->status_dev);
-  if (g->status_host) cudaFreeHost(g->status_host);
   cudaFree(g->shot_cand_offsets); cudaFree(g->shot_counts); cudaFree(g->shot_lrf);
   cudaFree(g->shot_runs);
   cudaFree(g->shot_frame32); cudaFree(g->shot_worklist); cudaFree(g->shot_pairs);
@@ -307,13 +306,15 @@ extern "C" int sf_grid_set_speculative(sf_grid* g, int32_t enable) {
   return SF_OK;
 }
 
+// The flag is read here, once, rather than copied to the host at the end of every call: a device-to-host copy between
+// the kernels of a repeated step costs more than the copy itself (the stream waits for the copy engine and back).
 extern "C" int sf_grid_poll(sf_grid* g, int32_t* status) {
   SF_REQUIRE(g != nullptr && status != nullptr, SF_ERR_ARG, "sf_grid_poll: null argument");
-  *status = g->status_host != nullptr ? *g->status_host : 0;
+  *status = 0;
+  if (g->status_dev != nullptr) SF_CUDA(cudaMemcpy(status, g->status_dev, sizeof(int32_t), cudaMemcpyDeviceToHost));
   if (*status != 0) {  // what was assumed does not hold: the next calls read everything back again
     g->sized = false;
     g->shot_entries_per_query = 0;
-    *g->status_host = 0;
     SF_CUDA(cudaMemset(g->status_dev, 0, sizeof(int32_t)));
   }
   return SF_OK;
@@ -345,8 +346,6 @@ static int reserve_points(sf_grid* g, const double* xyz, const double* normals, 
   if (g->status_dev == nullptr) {
     SF_CUDA(cudaMalloc(&g->status_dev, sizeof(int32_t)));
     SF_CUDA(cudaMemset(g->status_dev, 0, sizeof(int32_t)));
-    SF_CUDA(cudaHostAlloc(&g->status_host, sizeof(int32_t), cudaHostAllocDefault));
-    *g->status_host = 0;
   }
   return SF_OK;
 }
@@ -491,8 +490,6 @@ static int build_cells(sf_grid* g, const double* xyz, const double* normals, int
                                                     g->inv_perm, view, g->xyzc, g->nrm32);
   }
   SF_CUDA(cudaGetLastError());
-  if (check_box)  // the verdict, for sf_grid_poll
-    SF_CUDA(cudaMemcpyAsync(g->status_host, g->status_dev, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
   return SF_OK;
 }
 
@@ -512,6 +509,23 @@ extern "C" int sf_grid_permutation(const sf_grid* g, int32_t* perm_out, int32_t*
     SF_CUDA(cudaMemcpyAsync(perm_out, g->perm, g->n * sizeof(int32_t), cudaMemcpyDeviceToDevice, stream));
   if (inv_perm_out)
     SF_CUDA(cudaMemcpyAsync(inv_perm_out, g->inv_perm, g->n * sizeof(int32_t), cudaMemcpyDeviceToDevice, stream));
+  return SF_OK;
+}
+
+extern "C" int sf_grid_arrays(const sf_grid* g, double* pts_out, double* nrm_out, float* xyzc_out, float* nrm32_out,
+                              int32_t* cell_start_out, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  SF_REQUIRE(g != nullptr && g->n > 0, SF_ERR_ARG, "sf_grid_arrays: grid not built");
+  SF_REQUIRE(g->has_normals || (nrm_out == nullptr && nrm32_out == nullptr), SF_ERR_ARG,
+             "sf_grid_arrays: the grid was built without normals");
+  const auto copy = [&](void* dst, const void* src, size_t bytes) {
+    return dst != nullptr ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, stream) : cudaSuccess;
+  };
+  SF_CUDA(copy(pts_out, g->pts, g->n * sizeof(double4)));
+  SF_CUDA(copy(nrm_out, g->nrm, g->n * sizeof(double4)));
+  SF_CUDA(copy(xyzc_out, g->xyzc, g->n * sizeof(float4)));
+  SF_CUDA(copy(nrm32_out, g->nrm32, g->n * sizeof(float4)));
+  SF_CUDA(copy(cell_start_out, g->cell_start, (g->ncells + 1) * sizeof(int32_t)));
   return SF_OK;
 }
 

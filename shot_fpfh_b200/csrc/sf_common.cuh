@@ -130,7 +130,6 @@ struct sf_grid {
   int64_t sized_n = 0;         // ... this many points
   double sized_radius = 0.0;   // ... for this radius
   int32_t* status_dev = nullptr;   // 0 = fine; 1 = a point outside the assumed box; 2 = neighbour list too small
-  int32_t* status_host = nullptr;  // page-locked mirror, valid after the stream is synchronised
   // scratch of sf_shot_single_scale, kept between calls
   int64_t shot_q_capacity = 0;
   int64_t* shot_cand_offsets = nullptr;

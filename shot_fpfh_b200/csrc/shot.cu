@@ -1173,8 +1173,6 @@ extern "C" int sf_shot_single_scale(sf_grid* g, const double* queries, int64_t n
   int rc = launch_descriptor(g, queries, nq, radius, cand_offsets, counts, nbr, true, lrf, frame32, lrf_out != nullptr, min_nb,
                              normalize, out, out_is_f64, worklist + 1, worklist, status, stream, true);
   profile_mark(3, stream);
-  if (g->speculative && g->status_host != nullptr)  // the verdict of the device-side checks, for sf_grid_poll
-    SF_CUDA(cudaMemcpyAsync(g->status_host, g->status_dev, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
   if (rc == SF_OK && pairs_host != nullptr) {  // neighbour pairs found (logging / algorithmic-byte accounting)
     unsigned long long pairs = 0;
     int32_t deferred = 0;

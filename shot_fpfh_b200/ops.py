@@ -74,6 +74,25 @@ def grid_permutation(grid: Grid) -> tuple[torch.Tensor, torch.Tensor]:
     return perm, inv
 
 
+def grid_arrays(grid: Grid, normals: bool) -> dict[str, torch.Tensor]:
+    """Copies of the grid's cell-sorted arrays as CUDA tensors: pts (n, 4) float64, xyzc (n, 4) float32, cell_start
+    (ncells + 1) int32 and, when `normals` (the grid must have been built with them), nrm and nrm32."""
+    dev = require_cuda()
+    info = grid.info()
+    n, ncells = info["n"], info["ncells"]
+    out = {
+        "pts": torch.empty((n, 4), dtype=torch.float64, device=dev),
+        "xyzc": torch.empty((n, 4), dtype=torch.float32, device=dev),
+        "cell_start": torch.empty(ncells + 1, dtype=torch.int32, device=dev),
+    }
+    if normals:
+        out["nrm"] = torch.empty((n, 4), dtype=torch.float64, device=dev)
+        out["nrm32"] = torch.empty((n, 4), dtype=torch.float32, device=dev)
+    check(lib.sf_grid_arrays(grid.handle, ptr(out["pts"]), ptr(out.get("nrm")), ptr(out["xyzc"]), ptr(out.get("nrm32")),
+                             ptr(out["cell_start"]), stream_ptr()))
+    return out
+
+
 def voxel_subsample(xyz: torch.Tensor, voxel_size: float, want_members: bool = False):
     """
     Indices (int64, device) of one point per occupied voxel — `grid_subsampling` semantics, see csrc/subsample.cu.
