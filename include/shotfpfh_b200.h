@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SF_ABI_VERSION 14
+#define SF_ABI_VERSION 15
 
 #define SF_OK 0
 #define SF_ERR_CUDA 1     /* a CUDA runtime call or kernel launch failed */
@@ -329,6 +329,28 @@ int sf_match_rerank(const double* a_desc_dev, const int64_t* rows_a_dev, int64_t
  * || R a_i + t - b_i || <= threshold; a_dev / b_dev: the matched scan / reference keypoints, float64 (m,3). */
 int sf_ransac_count_inliers(const double* a_dev, const double* b_dev, int64_t m, const double* transforms_dev,
                             int64_t n_draws, double threshold, int32_t* counts_dev, void* stream);
+/* Adaptive RANSAC on the m matches (a_dev, b_dev: matched scan / reference keypoints, float64 (m,3), 3 <= m < 2^32);
+ * oracle/adaptive_ransac_oracle.py is the specification. Draw d picks three distinct matches from splitmix64 of
+ * seed * 0x9E3779B97F4A7C15 + 3d + s; a draw survives when every edge length of the triple agrees between the two
+ * clouds within edge_similarity (in (0, 1]), is fitted by Kabsch (eigh3 of H^T H; rejected when degenerate) and is
+ * valid when its own three pairs are inliers (|| R a + t - b || <= threshold, the predicate of
+ * sf_ransac_count_inliers). Draws run in batches of 2^20 (the last truncated to max_draws, in [1, 2^32 - 1]) until
+ * max_draws or until k 2^20 log1p(-(c/m)^3) <= log(1 - confidence) for the best count c. The winner is the valid draw
+ * with the most inliers, the lowest draw on ties. Outputs: transform_host[12] (rotation row-major, translation), its
+ * draw and count (-1 and 0 if no draw was valid), the draws run, the valid draws over all batches, and
+ * inlier_mask_dev (uint8[m]) = the winner's inliers. Two host synchronisations per batch; synchronises `stream`. */
+int sf_ransac_adaptive(const double* a_dev, const double* b_dev, int64_t m, double threshold, double edge_similarity,
+                       uint64_t seed, int64_t max_draws, double confidence, double* transform_host,
+                       int64_t* best_draw_host, int64_t* best_count_host, int64_t* draws_used_host, int64_t* valid_host,
+                       uint8_t* inlier_mask_dev, void* stream);
+/* One batch of the above, draws [first_draw, first_draw + n_draws) with n_draws <= 2^20, with what it produces:
+ * survivors_dev = the draws that pass the edge check, valid_draws_dev / transforms_dev (12 doubles each) / counts_dev =
+ * the valid draws, their transforms and inlier counts (each list in no particular order; buffers of n_draws entries).
+ * n_host[2] = {survivors, valid}. Synchronises `stream`. */
+int sf_ransac_adaptive_batch(const double* a_dev, const double* b_dev, int64_t m, double threshold,
+                             double edge_similarity, uint64_t seed, int64_t first_draw, int64_t n_draws,
+                             uint32_t* survivors_dev, uint32_t* valid_draws_dev, double* transforms_dev,
+                             int32_t* counts_dev, int64_t* n_host, void* stream);
 /* One ICP point-to-plane iteration (`icp_point_to_plane`, icp.py:157-182 with `solver_point_to_plane`,
  * core/solvers.py:34-48) on a grid built over the REFERENCE cloud with its normals and radius >= d_max: the scan
  * points are moved by transform_host (12 doubles, as above), each one's nearest reference point is found

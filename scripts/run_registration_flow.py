@@ -4,7 +4,7 @@ compute_descriptors, find_descriptors_matches, run_ransac, run_icp) through THIS
 NumPy arrays in and out at every stage, on a synthetic rigid pair (SURVEY.md 8d generator). BASELINE.json configs[4]
 names a 10M-point pair; the size is an argument:
 
-    python scripts/run_registration_flow.py [n_points] [fpfh] [voxel|iss] [pca|pca_raw]
+    python scripts/run_registration_flow.py [n_points] [fpfh] [voxel|iss] [pca|pca_raw] [adaptive]
 
 The keypoint selector is `voxel` (select_keypoints_subsampling, 3.75 spacings: the default) or `iss`
 (select_keypoints_iss, salient radius 5 spacings, non-max radius 3.75 spacings: far fewer keypoints, on salient points).
@@ -12,6 +12,8 @@ The normals are the synthetic surface's analytic ones (the default), or `pca`: c
 oriented by orient_normals (k = 10) towards the cloud's centroid and then negated, so that both clouds' normals point
 away from it, as the analytic ones do. `pca_raw` keeps compute_normals' signs (LAPACK's, a coin flip per point): it
 measures what sign noise does to matching.
+The coarse alignment is the reference's `ransac_on_matches` (10 000 draws of 4 matches), or with `adaptive`
+ransac_on_matches_adaptive (device-drawn 3-match hypotheses until 99.9 % confidence), same threshold.
 Prints wall-clock per stage and the error of the recovered transform against the known one. (`/root/reference` is not
 on the GPU box, so its `RegistrationPipeline` object cannot be run there; `dropin.install()` binds exactly these
 callables into it.)
@@ -36,11 +38,11 @@ from shot_fpfh_b200.descriptors import (  # noqa: E402
 )
 from shot_fpfh_b200.icp import icp_point_to_plane  # noqa: E402
 from shot_fpfh_b200.keypoint_selection import select_keypoints_iss, select_keypoints_subsampling  # noqa: E402
-from shot_fpfh_b200.matching import match_descriptors, ransac_on_matches  # noqa: E402
+from shot_fpfh_b200.matching import match_descriptors, ransac_on_matches, ransac_on_matches_adaptive  # noqa: E402
 
 
 def run(n: int, with_fpfh: bool = False, verbose: bool = True, keypoints: str = "voxel",
-        normals_from: str = "analytic") -> dict:
+        normals_from: str = "analytic", adaptive: bool = False) -> dict:
     times = {}
 
     def stage(name, fn):
@@ -93,13 +95,17 @@ def run(n: int, with_fpfh: bool = False, verbose: bool = True, keypoints: str = 
     import shot_fpfh_b200.matching.ransac as ransac_module
 
     ransac_module.rng = np.random.default_rng(seed=72)  # the reference's module-level generator (ransac.py:14)
-    ratio, coarse = stage("ransac_on_matches (10000 draws)", lambda: ransac_on_matches(
-        matches[0], matches[1], scan[scan_kp], ref[ref_kp], n_draws=10_000, distance_threshold=4 * s))
+    if adaptive:
+        ratio, coarse = stage("ransac_on_matches_adaptive", lambda: ransac_on_matches_adaptive(
+            matches[0], matches[1], scan[scan_kp], ref[ref_kp], distance_threshold=4 * s))
+    else:
+        ratio, coarse = stage("ransac_on_matches (10000 draws)", lambda: ransac_on_matches(
+            matches[0], matches[1], scan[scan_kp], ref[ref_kp], n_draws=10_000, distance_threshold=4 * s))
     fine, rms, _ = stage("icp_point_to_plane (<= 20 iters)", lambda: icp_point_to_plane(
         scan, ref, ref_normals, RigidTransform(coarse.rotation, coarse.translation), d_max=2 * s, voxel_size=3.75 * s,
         max_iter=20, rms_threshold=1e-9))
     out = {
-        "n_points": n, "keypoint_selector": keypoints, "normals": normals_from, "keypoints": (int(scan_kp.shape[0]), int(ref_kp.shape[0])), "matches": int(matches[0].shape[0]),
+        "n_points": n, "keypoint_selector": keypoints, "normals": normals_from, "adaptive_ransac": adaptive, "keypoints": (int(scan_kp.shape[0]), int(ref_kp.shape[0])), "matches": int(matches[0].shape[0]),
         "ransac_inlier_ratio": float(ratio),
         "coarse_rotation_error": float(np.abs(coarse.rotation - rot).max()),
         "fine_rotation_error": float(np.abs(fine.rotation - rot).max()),
@@ -116,4 +122,5 @@ if __name__ == "__main__":
     size = int(sys.argv[1]) if len(sys.argv) > 1 else 10_000_000
     words = sys.argv[2:]
     normals_from = "pca" if "pca" in words else ("pca_raw" if "pca_raw" in words else "analytic")
-    run(size, with_fpfh="fpfh" in words, keypoints="iss" if "iss" in words else "voxel", normals_from=normals_from)
+    run(size, with_fpfh="fpfh" in words, keypoints="iss" if "iss" in words else "voxel", normals_from=normals_from,
+        adaptive="adaptive" in words)

@@ -10,11 +10,11 @@ from __future__ import annotations
 
 import ctypes
 import os
-from ctypes import POINTER, c_char_p, c_double, c_float, c_int32, c_int64, c_void_p
+from ctypes import POINTER, c_char_p, c_double, c_float, c_int32, c_int64, c_uint64, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "csrc", "libshotfpfh_b200.so")
-ABI_VERSION = 14
+ABI_VERSION = 15
 
 SF_OK, SF_ERR_CUDA, SF_ERR_ARG, SF_ERR_CAPACITY = 0, 1, 2, 3
 
@@ -92,6 +92,10 @@ def _load() -> ctypes.CDLL:
             c_void_p,
         ],
         "sf_ransac_count_inliers": [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_double, c_void_p, c_void_p],
+        "sf_ransac_adaptive": [c_void_p, c_void_p, c_int64, c_double, c_double, c_uint64, c_int64, c_double, p_f64,
+                               p_i64, p_i64, p_i64, p_i64, c_void_p, c_void_p],
+        "sf_ransac_adaptive_batch": [c_void_p, c_void_p, c_int64, c_double, c_double, c_uint64, c_int64, c_int64,
+                                     c_void_p, c_void_p, c_void_p, c_void_p, p_i64, c_void_p],
         "sf_icp_plane_step": [c_void_p, c_void_p, c_int64, p_f64, c_double, p_f64, c_void_p, c_void_p],
         "sf_fpfh_row_stride": [c_int32, POINTER(c_int32)],
         "sf_fpfh_block_begin": [c_void_p, c_double, c_int64, c_int64, c_void_p, p_i64, c_void_p],
@@ -118,7 +122,7 @@ lib = _load()
 EXPORTS = (
     "sf_last_error sf_abi_version sf_grid_create sf_grid_destroy sf_grid_build sf_grid_info sf_grid_build_in_box sf_grid_geometry sf_grid_set_speculative sf_grid_poll sf_grid_permutation sf_grid_arrays "
     "sf_radius_count sf_radius_fill sf_voxel_subsample sf_knn sf_pca_normals sf_iss_saliency sf_iss_select sf_orient_normals sf_shot_lrf sf_shot_descriptor sf_shot_single_scale sf_shot_last_deferred sf_profile_enable sf_profile_read sf_spfh sf_fpfh sf_fpfh_cloud sf_fpfh_row_stride sf_fpfh_block_begin sf_fpfh_block_spfh sf_fpfh_block_rows sf_nonempty_rows sf_match_certify sf_match_exhaustive sf_match_exhaustive_topk sf_match_pack "
-    "sf_match_topk sf_topk_merge sf_nearest_merge sf_match_rerank sf_ransac_count_inliers sf_icp_plane_step sf_rows_compact_count sf_rows_compact_fill "
+    "sf_match_topk sf_topk_merge sf_nearest_merge sf_match_rerank sf_ransac_count_inliers sf_ransac_adaptive sf_ransac_adaptive_batch sf_icp_plane_step sf_rows_compact_count sf_rows_compact_fill "
     "sf_host_expand_rows_begin sf_host_widen_begin sf_host_copy_begin sf_host_advise_huge sf_host_wait"
 ).split()
 

@@ -2,7 +2,7 @@
 
 from .filters import FilterFunction, left_median_filter, quantile_filter, threshold_filter
 from .matching import basic_matching, double_matching_with_rejects, match_descriptors
-from .ransac import ransac_on_matches
+from .ransac import ransac_on_matches, ransac_on_matches_adaptive
 
 __all__ = [
     "FilterFunction",
@@ -13,4 +13,5 @@ __all__ = [
     "basic_matching",
     "double_matching_with_rejects",
     "ransac_on_matches",
+    "ransac_on_matches_adaptive",
 ]

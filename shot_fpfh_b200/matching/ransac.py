@@ -8,6 +8,11 @@ with the largest count. The cost is the n_draws x n_matches count: that runs on 
 generator, seeded and advanced the same way, so the same draws, taken from its raw stream in one vectorised pass
 (`replay_choices`) — and the n_draws 3x3 SVDs are one batched host call.
 The winning transform is then refitted with the scalar solver, i.e. exactly the reference's arithmetic.
+
+`ransac_on_matches_adaptive` is this package's own coarse alignment for match sets with few inliers, where 10 000
+draws of 4 matches rarely contain an all-inlier sample (probability w^4 per draw at inlier ratio w): device-drawn
+3-match samples, an edge-length check that rejects most outlier triples before any fit, and as many draws as the
+confidence asks for (`sf_ransac_adaptive`, csrc/registration.cu; specification: oracle/adaptive_ransac_oracle.py).
 """
 
 from __future__ import annotations
@@ -150,3 +155,66 @@ def ransac_on_matches(
     best_transform = solver_point_to_point(matched_scan[draws[best]], matched_ref[draws[best]])
     best_transform.normalize_rotation()
     return best_n_inliers / n_matches, best_transform
+
+
+def ransac_on_matches_adaptive(
+    scan_descriptors_indices: np.ndarray,
+    ref_descriptors_indices: np.ndarray,
+    scan_keypoints: npt.NDArray[np.float64],
+    ref_keypoints: npt.NDArray[np.float64],
+    distance_threshold: float = 1,
+    confidence: float = 0.999,
+    max_draws: int = 1 << 24,
+    edge_similarity: float = 0.9,
+    seed: int = 0,
+    verbose: bool = False,
+) -> tuple[float, RigidTransform]:
+    """
+    Adaptive RANSAC on the matches, on the device. Returns (share of the matches that are inliers of the best
+    hypothesis, its transform refitted on all those inliers by `solver_point_to_point`, rotation normalised), as
+    `ransac_on_matches` does.
+
+    Draw d takes three distinct matches from a counter-based generator seeded by `seed`; it is fitted only if every
+    edge of the triple has the same length in both clouds within `edge_similarity` (shorter >= edge_similarity x
+    longer), and kept only if its own three matches are inliers of its fit. A match is an inlier when
+    ||R a + t - b|| <= distance_threshold. Draws run in batches of 2^20 until `max_draws`, or until the chance that
+    every draw so far missed an all-inlier triple, (1 - (c / m)^3)^draws for the best count c, is at most
+    1 - confidence. The best hypothesis has the most inliers; ties go to the earliest draw. The result depends only
+    on the inputs and `seed`.
+
+    Raises ValueError on fewer than 3 or more than 2^32 - 1 matches, non-finite matched keypoints,
+    distance_threshold <= 0, confidence outside (0, 1), edge_similarity outside (0, 1] or max_draws outside
+    [1, 2^32 - 1]; RuntimeError when no draw passes the checks (e.g. every triple collinear).
+    """
+    from .. import ops
+    from ..device import upload
+
+    n_matches = len(scan_descriptors_indices)
+    if len(ref_descriptors_indices) != n_matches:
+        raise ValueError(f"{n_matches} scan indices but {len(ref_descriptors_indices)} reference indices")
+    if not 3 <= n_matches <= 0xFFFFFFFF:
+        raise ValueError(f"adaptive RANSAC needs 3 to 2^32 - 1 matches, got {n_matches}")
+    if not (np.isfinite(distance_threshold) and distance_threshold > 0):
+        raise ValueError(f"distance_threshold must be positive and finite, got {distance_threshold}")
+    if not 0.0 < confidence < 1.0:
+        raise ValueError(f"confidence must lie in (0, 1), got {confidence}")
+    if not 0.0 < edge_similarity <= 1.0:
+        raise ValueError(f"edge_similarity must lie in (0, 1], got {edge_similarity}")
+    if not 1 <= max_draws <= 0xFFFFFFFF:
+        raise ValueError(f"max_draws must lie in [1, 2^32 - 1], got {max_draws}")
+    matched_scan = np.ascontiguousarray(scan_keypoints[scan_descriptors_indices], dtype=np.float64)
+    matched_ref = np.ascontiguousarray(ref_keypoints[ref_descriptors_indices], dtype=np.float64)
+    if not (np.isfinite(matched_scan).all() and np.isfinite(matched_ref).all()):
+        raise ValueError("the matched keypoints must be finite")
+    out = ops.ransac_adaptive(upload(matched_scan), upload(matched_ref), float(distance_threshold),
+                              float(edge_similarity), int(seed), int(max_draws), float(confidence))
+    if out["valid"] == 0:
+        raise RuntimeError(f"adaptive RANSAC: none of {out['draws_used']} draws passed the edge and fit checks "
+                           "(collinear or inconsistent matches)")
+    if verbose:
+        logging.info(f"Best draw: #{out['best_draw']} with {out['best_count']} inliers out of {n_matches} matches "
+                     f"({out['draws_used']} draws, {out['valid']} valid)")
+    inliers = out["mask"].cpu().numpy().astype(bool)
+    best_transform = solver_point_to_point(matched_scan[inliers], matched_ref[inliers])
+    best_transform.normalize_rotation()
+    return out["best_count"] / n_matches, best_transform

@@ -500,6 +500,55 @@ def ransac_count_inliers(matched_scan: torch.Tensor, matched_ref: torch.Tensor, 
     return counts
 
 
+def ransac_adaptive(matched_scan: torch.Tensor, matched_ref: torch.Tensor, threshold: float, edge_similarity: float,
+                    seed: int, max_draws: int, confidence: float) -> dict:
+    """
+    Adaptive RANSAC (sf_ransac_adaptive) on (m, 3) float64 device tensors: {"transform": float64 (12,) host array
+    (rotation row-major, translation), "best_draw", "best_count", "draws_used", "valid": ints, "mask": uint8 (m,)
+    device tensor of the winner's inliers}; best_draw is -1 and valid 0 when no draw passed the checks.
+    """
+    import numpy as np
+
+    m = int(matched_scan.shape[0])
+    assert matched_scan.dtype == torch.float64 and matched_ref.shape == matched_scan.shape
+    transform = np.zeros(12, dtype=np.float64)
+    counters = [ctypes.c_int64() for _ in range(4)]
+    mask = torch.empty(m, dtype=torch.uint8, device=matched_scan.device)
+    check(lib.sf_ransac_adaptive(ptr(matched_scan), ptr(matched_ref), m, float(threshold), float(edge_similarity),
+                                 int(seed) & 0xFFFFFFFFFFFFFFFF, int(max_draws), float(confidence),
+                                 transform.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
+                                 *(ctypes.byref(c) for c in counters), ptr(mask), stream_ptr()))
+    best_draw, best_count, draws_used, valid = (c.value for c in counters)
+    return {"transform": transform, "best_draw": best_draw, "best_count": best_count, "draws_used": draws_used,
+            "valid": valid, "mask": mask}
+
+
+def ransac_adaptive_batch(matched_scan: torch.Tensor, matched_ref: torch.Tensor, threshold: float,
+                          edge_similarity: float, seed: int, first_draw: int, n_draws: int) -> dict:
+    """One batch of sf_ransac_adaptive (sf_ransac_adaptive_batch): {"survivors": uint32 as int64 device tensor of the
+    draws that pass the edge check, "valid_draws", "transforms" (V, 12), "counts": the valid draws, their transforms
+    and inlier counts}, each sorted by draw index."""
+    m = int(matched_scan.shape[0])
+    assert matched_scan.dtype == torch.float64 and matched_ref.shape == matched_scan.shape
+    dev = matched_scan.device
+    survivors = torch.empty(n_draws, dtype=torch.int32, device=dev)
+    valid_draws = torch.empty(n_draws, dtype=torch.int32, device=dev)
+    transforms = torch.empty((n_draws, 12), dtype=torch.float64, device=dev)
+    counts = torch.empty(n_draws, dtype=torch.int32, device=dev)
+    n = (ctypes.c_int64 * 2)()
+    check(lib.sf_ransac_adaptive_batch(ptr(matched_scan), ptr(matched_ref), m, float(threshold),
+                                       float(edge_similarity), int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_draw),
+                                       int(n_draws), ptr(survivors), ptr(valid_draws), ptr(transforms), ptr(counts),
+                                       n, stream_ptr()))
+
+    def as_draws(t: torch.Tensor) -> torch.Tensor:  # uint32 bits -> int64
+        return t.to(torch.int64) & 0xFFFFFFFF
+
+    order = torch.argsort(as_draws(valid_draws[: n[1]]))
+    return {"survivors": torch.sort(as_draws(survivors[: n[0]])).values, "valid_draws": as_draws(valid_draws[: n[1]])[order],
+            "transforms": transforms[: n[1]][order], "counts": counts[: n[1]][order]}
+
+
 def icp_plane_step(ref_grid: Grid, scan: torch.Tensor, transform_row, d_max: float, want_nearest: bool = False):
     """
     One point-to-plane ICP iteration's sums (sf_icp_plane_step): float64 (29,) host array = 21 entries of g^T g

@@ -89,6 +89,37 @@ def rigid_pair(
     return ref, ref_normals, perm, rot, _PAIR_TRANSLATION.copy()
 
 
+def corrupted_matches(
+    n: int, inlier_ratio: float, noise: float = 0.0, seed: int = 0
+) -> tuple[
+    npt.NDArray[np.float64],
+    npt.NDArray[np.float64],
+    npt.NDArray[np.int64],
+    npt.NDArray[np.int64],
+    npt.NDArray[np.float64],
+    npt.NDArray[np.float64],
+]:
+    """
+    A registration pair with n matches of known quality, for coarse-alignment tests: the bumpy sphere of n points and
+    its `rigid_pair` copy, with isotropic Gaussian noise of standard deviation `noise` added to the reference points.
+    Match i pairs scan point i with its true counterpart for round(inlier_ratio * n) randomly chosen i and with a
+    uniformly drawn reference point otherwise. Returns (scan, ref, scan_idx, ref_idx, rotation, translation), with
+    ref ~ (scan @ rotation.T + translation)[perm].
+    """
+    scan, directions = bumpy_sphere(n, seed=seed)
+    ref, _, perm, rot, trans = rigid_pair(scan, directions, perm_seed=seed + 1)
+    rng = np.random.default_rng(seed + 2)
+    if noise > 0.0:
+        ref = ref + rng.normal(scale=noise, size=ref.shape)
+    inverse = np.empty(n, dtype=np.int64)
+    inverse[perm] = np.arange(n)
+    scan_idx = np.arange(n, dtype=np.int64)
+    ref_idx = rng.integers(0, n, size=n)
+    correct = rng.permutation(n)[: int(round(inlier_ratio * n))]
+    ref_idx[correct] = inverse[correct]
+    return scan, np.ascontiguousarray(ref), scan_idx, ref_idx, rot, trans
+
+
 def voxel_first_point_queries(
     points: npt.NDArray[np.float64], voxel_size: float
 ) -> npt.NDArray[np.int64]:
